@@ -23,6 +23,10 @@ all-gather's vector against NCCL's; `cpu_baseline` = the reference implementatio
 (oracle/_ref, staged by oracle/Makefile) on the box's host cores.
 
 `--impl reference` times that CPU implementation alone, on the same config/metric.
+
+`--dump-outputs DIR` writes the lnL vector of the last timed step (what the caller of the step
+receives: at N > 1 the gathered vector of all ranks) to DIR/lnl.npy in float64, so that two builds
+run with the same arguments, and therefore the same seeded theta, can be compared row for row.
 """
 import argparse
 import gc
@@ -45,6 +49,7 @@ LATENCY_CONFIG = 2     # configs[1]: the UltraNest ndraw = 4096 call, reported a
 LATENCY_BATCH = 4096
 STRESS_TOTAL = 10_000_000  # configs[4]: 1e7 theta x 1e4 epochs x 3 planets over all ranks
 NOMINAL_RATE = 4.5e6   # lnL/s/GPU on config 3: only used to size the batch deterministically
+DUMP_BYTES = 64_000_000  # --dump-outputs: at most this much in all
 
 
 def batch_for(steps):
@@ -60,6 +65,21 @@ def batch_for(steps):
 def algorithmic_flops(n_epochs, n_planets, drift_order, mean_iters):
     """SURVEY.md 8(d): F = N [K (51 + 46 I) + 48 + 2 d] FP64 flops per lnL."""
     return n_epochs * (n_planets * (51.0 + 46.0 * mean_iters) + 48.0 + 2.0 * drift_order)
+
+
+def dump_outputs(dirpath, lnl):
+    """Write the last timed step's lnL vector as DIR/lnl.npy (float64).  A vector larger than half
+    of DUMP_BYTES (N = 8 at the largest batch) is replaced by a fixed seeded sample of a quarter of
+    that size, with the rows' positions in DIR/lnl_rows.npy (float64, exact)."""
+    lnl = np.ascontiguousarray(lnl, dtype=np.float64)
+    os.makedirs(dirpath, exist_ok=True)
+    out = {"lnl": lnl}
+    if lnl.nbytes > DUMP_BYTES // 2:
+        rows = np.sort(np.random.default_rng(0).choice(lnl.size, DUMP_BYTES // 32, replace=False))
+        out = {"lnl": lnl[rows], "lnl_rows": rows.astype(np.float64)}
+    for name, arr in out.items():
+        np.save(os.path.join(dirpath, name + ".npy"), arr)
+    return sorted(out)
 
 
 def workload_config(case, batch, world):
@@ -539,7 +559,11 @@ def main():
                     help="multi-GPU: the all-gather fused into the likelihood launch over NVLink "
                          "symmetric memory (peer stores + completion flags; default), the same with "
                          "a symmetric-memory barrier, or NCCL all_gather")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the lnL vector of the last timed step to DIR/lnl.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -701,7 +725,7 @@ def main():
     for k in range(K):
         flush.zero_()  # L2 flush, outside the per-step events
         ev[k][0].record()
-        step()
+        last = step()
         ev[k][1].record()
         if inner_events:
             kms.append(model.last_kernel_ms())
@@ -709,6 +733,8 @@ def main():
                 wms.append(model.last_gather_wait_ms())
     ranks.barrier()
     t_wall = time.perf_counter() - t_wall
+    if args.dump_outputs and rank == 0:  # before the end-to-end calls re-use the buffers
+        dump_outputs(args.dump_outputs, last.cpu().numpy())
     dev_ms = float(sum(a.elapsed_time(b) for a, b in ev))
     launches = model.launch_count() - launches0
     if not inner_events:

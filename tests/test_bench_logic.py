@@ -67,3 +67,20 @@ def test_parity_verdict_passes_fails_and_classifies_cap_rows():
     assert not bench.parity_verdict(sets, bad, want, "reference", classify=lambda row: (0, 0))[1]
     rep, ok = bench.parity_verdict(sets, bad, want, "reference", classify=lambda row: (1, 0))
     assert ok and rep["sets"]["ecc_0.97_1.00"]["cap_rows"][0]["row"] == 11
+
+
+def test_dump_outputs_writes_float64_within_the_size_cap(tmp_path, monkeypatch):
+    lnl = np.random.default_rng(1).uniform(-1e5, -1e4, 4096)
+    assert bench.dump_outputs(str(tmp_path / "a"), lnl) == ["lnl"]
+    back = np.load(tmp_path / "a" / "lnl.npy")
+    assert back.dtype == np.float64 and np.array_equal(back, lnl)
+    # a vector over the cap: the same seeded sample of rows every time, with the rows' positions
+    monkeypatch.setattr(bench, "DUMP_BYTES", 64_000)
+    big = np.arange(bench.DUMP_BYTES // 8 + 10, dtype=np.float64)
+    for d in ("b", "c"):
+        assert bench.dump_outputs(str(tmp_path / d), big) == ["lnl", "lnl_rows"]
+    files = [tmp_path / d / f"{n}.npy" for d in ("b", "c") for n in ("lnl", "lnl_rows")]
+    assert sum(f.stat().st_size for f in files[:2]) <= bench.DUMP_BYTES
+    got, rows = np.load(files[0]), np.load(files[1])
+    assert got.dtype == rows.dtype == np.float64 and np.array_equal(got, big[rows.astype(np.int64)])
+    assert np.array_equal(np.load(files[2]), got) and np.all(np.diff(rows) > 0)
