@@ -104,6 +104,10 @@ SYMBOLS = {
     "rvl_transform_loglike_dev": (c_int32, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p,
                                             c_void_p]),
     "rvl_trueanomaly": (c_int32, [c_void_p, _dp, c_int32, c_double, _dp, c_int32, c_double]),
+    "rvl_kepler_rv": (c_int32, [c_void_p, c_void_p, c_int64, c_void_p, c_int32, ctypes.c_uint32,
+                                c_void_p, c_void_p, POINTER(c_uint64)]),
+    "rvl_kepler_rv_dev": (c_int32, [c_void_p, c_void_p, c_int64, c_void_p, c_int32, ctypes.c_uint32,
+                                    c_void_p, c_void_p, c_void_p, c_void_p]),
     "rvl_counters": (c_int32, [c_void_p, POINTER(rvl_counters_t)]),
     "rvl_reset_counters": (c_int32, [c_void_p]),
     "rvl_last_kernel_ms": (c_int32, [c_void_p, _dp]),

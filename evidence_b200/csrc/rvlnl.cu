@@ -3,7 +3,8 @@
 //
 // Reference path replaced (paths relative to the reference checkout):
 //   evidence/rvmodel/__init__.py:157-219  RVModel.log_likelihood      -> rv_lnl_kernel
-//   evidence/rvmodel/__init__.py:343-463  kep_rv / modelk             -> point_setup + solve_planet
+//   evidence/rvmodel/__init__.py:343-463  kep_rv / modelk             -> point_setup + solve_planet;
+//                                                                       at caller times: kepler_rv_kernel
 //   evidence/rvmodel/trueanomaly.c:8-41   trueanomaly()               -> solve_planet / trueanomaly_kernel
 //   evidence/rvmodel/__init__.py:222-273  drift                       -> epoch term of rv_lnl_kernel
 //   evidence/rvmodel/__init__.py:59-80    BaseModel.logL              -> epoch term + slice reduce
@@ -1223,6 +1224,115 @@ __global__ void trueanomaly_kernel(const double *M, int n, double ecc, double *n
     }
 }
 
+// ---- model velocity curves at caller times: kep_rv / modelk (:343-463) --------------------------
+// One warp per work item = (point b, group g of 32*U consecutive times); lane l, slot u holds time
+// g*32*U + u*32 + l, the lane <-> epoch map of the likelihood kernel, so every lane shares the
+// eccentricity and the Newton trips stay warp-uniform.  The per-point constants come from
+// point_prepare_kernel (d_consts, [B][wstride]); the item copies the planet blocks into the warp's
+// shared block and runs the likelihood kernel's solve_planet on them, planet after planet in
+// planet order, each solve adding its velocity to the lane's sum exactly as item_epochs does.  Each
+// output element is computed by one lane with no reduction across items: a row's curve does not
+// depend on the batch it came in.
+//   Padding of a point's last group: a slot past T repeats the lane's slot 0 (the last time when
+// that is past T too), so a lane whose second slot is padding ran two identical solves per planet
+// and its cap hits are exactly twice the live ones.
+struct CurveArgs {
+    const rvl_model_desc *model;    // device copy
+    const double *theta;            // [B][ndim]
+    const double *consts;           // [B][wstride]
+    const double *times;            // [T]
+    double *out;                    // [B][T]
+    uint32_t *invalid;              // [B] or NULL
+    unsigned long long *cap_hits;   // or NULL
+    long long nitems;               // B * G
+    int T, G, K, ndim, wstride, itmax;
+    uint32_t mask;
+    double tol;
+};
+
+// RVL_CURVE_MINB: resident 256-thread blocks per SM asked of ptxas (1: no register cap, 116
+// registers, no spills; 3: 80 registers with a few spilled bytes)
+#ifndef RVL_CURVE_MINB
+#define RVL_CURVE_MINB 1
+#endif
+template <int U>
+__global__ void __launch_bounds__(256, RVL_CURVE_MINB) kepler_rv_kernel(const CurveArgs a)
+{
+    static_assert(U == 2, "cap-hit accounting of the padding assumes two slots per lane");
+    __shared__ __align__(16) double s_pc[8][RVL_MAX_PLANETS * kPlanetStride];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    double *wc = s_pc[warp];
+    const uint32_t a_wc = smem_u32(wc);
+    const rvl::KTab kt = rvl::load_ktab_pinned();
+    const int K = a.K, T = a.T, G = a.G;
+    // the launch-wide conditions of the lean Newton loop (item_epochs)
+    const bool lean_ok = __double2hiint(a.tol) < rvl::kHiFinal && a.itmax >= 2;
+    int caps = 0;
+    const long long nw = (long long)gridDim.x * (blockDim.x >> 5);
+    for (long long it = (long long)blockIdx.x * (blockDim.x >> 5) + warp; it < a.nitems; it += nw) {
+        const long long b = it / G;
+        const int g = (int)(it - b * G);
+        const double *row = a.theta + b * a.ndim;
+        // validity of planet `lane`, the arithmetic of point_setup (:425-439)
+        bool bad = false;
+        if (lane < K) {
+            const rvl_planet_desc &pl = a.model->planet[lane];
+            if (pl.ecc_mode != RVL_ECC_DIRECT) {
+                const double c = par_of(pl.e1, row), s = par_of(pl.e2, row);
+                double e = rvl::add(rvl::mul(c, c), rvl::mul(s, s));
+                if (pl.ecc_mode == RVL_ECC_ECOS_ESIN) e = sqrt(e);
+                bad = e > 1.0;
+            }
+        }
+        const uint32_t badm = __ballot_sync(kFull, bad);
+        if (g == 0 && lane == 0 && a.invalid) a.invalid[b] = badm;
+        const bool valid = (badm & a.mask) == 0u;
+
+        __syncwarp();
+        const double *src = a.consts + b * a.wstride;
+        for (int i = lane; i < K * kPlanetStride; i += 32) wc[i] = __ldg(src + i);
+        __syncwarp();
+
+        const int j0 = g * 32 * U + lane;
+        double t[U], rv[U];
+        int it_l[U];
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            const int j = j0 + u * 32;
+            t[u] = T > 0 ? __ldg(a.times + (j < T ? j : (j0 < T ? j0 : T - 1))) : 0.0;
+            rv[u] = valid ? 0.0 : __longlong_as_double(0x7ff8000000000000LL);  // NaN row
+            it_l[u] = 0;
+        }
+        int cap_l = 0;
+        if (valid) {
+            for (int p = 0; p < K; ++p) {
+                if (!((a.mask >> p) & 1u)) continue;
+                const uint32_t pc = a_wc + (uint32_t)(p * kPlanetStride) * 8u;
+                // the lean loop needs every |M| of the item inside the fast sin/cos range (the
+                // prepare pass decided that for the data's epochs, not for these times)
+                const double nmot = lds_f64(pc), M0 = lds_f64(pc + 8), ec = lds_f64(pc + 16),
+                             epoch = lds_f64(pc + 48);
+                bool in_range = ec >= -0.99;
+#pragma unroll
+                for (int u = 0; u < U; ++u)
+                    in_range = in_range &&
+                               fabs(rvl::mean_anomaly(nmot, t[u], epoch, M0)) < 0.99 * rvl::kTrigFastMax;
+                const bool lean = lean_ok && __all_sync(kFull, in_range);
+                solve_planet<0, U>(kt, t, pc, a.tol, a.itmax, rv, it_l, cap_l, lean);
+            }
+        }
+        double *o = a.out + b * (long long)T;
+#pragma unroll
+        for (int u = 0; u < U; ++u)
+            if (j0 + u * 32 < T) o[j0 + u * 32] = rv[u];
+        caps += j0 + 32 < T ? cap_l : (j0 < T ? cap_l / 2 : 0);
+    }
+    if (a.cap_hits) {
+        const unsigned n = __reduce_add_sync(kFull, (unsigned)caps);
+        if (lane == 0 && n) atomicAdd(a.cap_hits, (unsigned long long)n);
+    }
+}
+
 // ---- register-resident DFMA loop: the FP64 roofline denominator -------------------------------
 template <int R>
 __global__ void __launch_bounds__(1024) dfma_peak_kernel(double *out, int iters, double, double b)
@@ -1301,6 +1411,13 @@ struct rvl_handle {
     int *d_flags = nullptr;
     unsigned long long *d_counters = nullptr;  // 3
     unsigned int *d_work = nullptr;            // sm_count + 1 (queues, finished-block counter)
+    // rvl_kepler_rv (host buffers): times, curves [B][T], invalid bits, cap-hit counter
+    double *d_curve_t = nullptr, *d_curve = nullptr;
+    size_t cap_curve_t = 0, cap_curve = 0;
+    uint32_t *d_curve_inv = nullptr;
+    long long cap_curve_inv = 0;
+    unsigned long long *d_curve_caps = nullptr;
+    int curve_blocks_per_sm = 0;  // resident blocks of kepler_rv_kernel (0: not asked yet)
 
     // options
     int opt_variant = 0, opt_slices = 0, opt_warps = 0, opt_timing = 0, opt_zero_copy = 1, opt_ilp = 0, opt_min_chunks = 8, opt_items_per_warp = 4;
@@ -1544,13 +1661,19 @@ const char *plan_core(const PlanIn &in, long long B, Plan &pl)
     return nullptr;
 }
 
+// doubles of per-point constants (point_setup's layout; +1: the lean flag)
+int consts_stride(const rvl_model_desc &m)
+{
+    return (m.n_planets * kPlanetStride + 2 * m.n_inst + 4 + m.n_linpar + 1 + 1) & ~1;
+}
+
 int make_plan(rvl_t *h, long long B, Plan &pl)
 {
     const rvl_model_desc &m = h->model;
     PlanIn in{};
     in.Ctot = (h->N + 31) / 32;  // (the columns themselves are padded further: see rvl_set_data)
     in.ncol = h->ncol;
-    in.wstride = (m.n_planets * kPlanetStride + 2 * m.n_inst + 4 + m.n_linpar + 1 + 1) & ~1;  // (+1: the lean flag)
+    in.wstride = consts_stride(m);
     in.wblock = in.wstride + ((m.ndim + 1) & ~1);
     // epochs per lane in flight: 4 (512 threads, 128 registers) when every warp has a long queue of
     // whole points AND a point is long enough to amortise its setup over the 16 warps per SM left --
@@ -1684,6 +1807,48 @@ int enqueue_transform(rvl_t *h, const double *dU, long long B, double *dTheta, c
     const int tb = 256;
     prior_transform_kernel<<<(unsigned)((total + tb - 1) / tb), tb, 0, st>>>(
         h->d_priors, h->d_tables, dU, dTheta, total, h->prior_ndim);
+    CU(h, cudaGetLastError());
+    ++h->launches;
+    return RVL_OK;
+}
+
+// Model velocity curves, device pointers: the prepare pass derives every point's constants into
+// d_consts, then kepler_rv_kernel evaluates them at the caller's times.  rvl_counters untouched.
+int enqueue_kepler_rv(rvl_t *h, const double *dTheta, long long B, const double *dTimes, int T,
+                      uint32_t mask, double *dOut, uint32_t *dInvalid, unsigned long long *dCaps,
+                      cudaStream_t st)
+{
+    if (!h->have_model) return fail(h, RVL_ESTATE, "set the model first");
+    const rvl_model_desc &m = h->model;
+    if (m.n_planets < 32 && (mask >> m.n_planets) != 0u)
+        return fail(h, RVL_EINVAL, "planet_mask names a planet the model does not have");
+    if (B <= 0) return RVL_OK;
+    const int wstride = consts_stride(m);
+    int rc = ensure_partial(h, B, 0, 0, /*prepare=*/true, wstride);
+    if (rc) return rc;
+    const int wpb = 8;  // warps (= points) per block
+    point_prepare_kernel<<<(unsigned)((B + wpb - 1) / wpb), wpb * 32, 0, st>>>(
+        h->d_model, nullptr, nullptr, nullptr, const_cast<double *>(dTheta), h->d_consts, h->d_flags,
+        B, wstride, h->tlo, h->thi);
+    CU(h, cudaGetLastError());
+    ++h->launches;
+    constexpr int U = 2, kThreads = 256;
+    if (!h->curve_blocks_per_sm) {
+        int n = 0;
+        CU(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kepler_rv_kernel<U>, kThreads, 0));
+        h->curve_blocks_per_sm = std::max(1, n);
+    }
+    CurveArgs a{};
+    a.model = h->d_model; a.theta = dTheta; a.consts = h->d_consts; a.times = dTimes; a.out = dOut;
+    a.invalid = dInvalid; a.cap_hits = dCaps;
+    // T == 0: one item per point that only writes the invalid bits
+    a.T = T; a.G = T > 0 ? (T + 32 * U - 1) / (32 * U) : 1; a.mask = T > 0 ? mask : 0u;
+    a.K = m.n_planets; a.ndim = m.ndim; a.wstride = wstride; a.itmax = m.itmax; a.tol = m.tol;
+    a.nitems = B * (long long)a.G;
+    const long long wpb2 = kThreads / 32;
+    const long long blocks = std::min<long long>((a.nitems + wpb2 - 1) / wpb2,
+                                                 (long long)h->sm_count * h->curve_blocks_per_sm);
+    kepler_rv_kernel<U><<<(unsigned)blocks, kThreads, 0, st>>>(a);
     CU(h, cudaGetLastError());
     ++h->launches;
     return RVL_OK;
@@ -2076,6 +2241,7 @@ void rvl_destroy(rvl_t *h)
     cudaFree(h->d_partial); cudaFree(h->d_flags); cudaFree(h->d_counters); cudaFree(h->d_work);
     cudaFree(h->d_consts); cudaFree(h->d_arrive); cudaFree(h->d_trace);
     cudaFree(h->d_gconsts); cudaFree(h->d_ready);
+    cudaFree(h->d_curve_t); cudaFree(h->d_curve); cudaFree(h->d_curve_inv); cudaFree(h->d_curve_caps);
     if (h->pin_in) cudaFreeHost(h->pin_in);
     if (h->pin_out) cudaFreeHost(h->pin_out);
     if (h->pin_out2) cudaFreeHost(h->pin_out2);
@@ -2420,6 +2586,72 @@ int rvl_trueanomaly(rvl_t *h, const double *M, int32_t n, double ecc, double *nu
     if (e != cudaSuccess) return fail(h, RVL_ECUDA, std::string("rvl_trueanomaly: ") + cudaGetErrorString(e));
     if (e2 != cudaSuccess) return fail(h, RVL_ECUDA, std::string("rvl_trueanomaly: ") + cudaGetErrorString(e2));
     return cap ? -1 : 0;  // same 0 / -1 convention as trueanomaly.c:32-40
+}
+
+int rvl_kepler_rv_dev(rvl_t *h, const double *dTheta, int64_t B, const double *dTimes, int32_t T,
+                      uint32_t planet_mask, double *dOut, uint32_t *dInvalid, uint64_t *dCapHits,
+                      void *stream)
+{
+    if (!h) return RVL_EINVAL;
+    if (!h->kids.empty()) return fail(h, RVL_EINVAL, "device-pointer entry points need a single-device handle");
+    if (B < 0 || T < 0 || (B > 0 && (!dTheta || (T > 0 && (!dTimes || !dOut)))))
+        return fail(h, RVL_EINVAL, "bad arguments");
+    DevGuard g(h->device);
+    return enqueue_kepler_rv(h, dTheta, B, dTimes, T, planet_mask, dOut, dInvalid,
+                             reinterpret_cast<unsigned long long *>(dCapHits), (cudaStream_t)stream);
+}
+
+int rvl_kepler_rv(rvl_t *h, const double *Theta, int64_t B, const double *times, int32_t T,
+                  uint32_t planet_mask, double *out, uint32_t *invalid, uint64_t *cap_hits)
+{
+    if (!h) return RVL_EINVAL;
+    if (B < 0 || T < 0 || (B > 0 && (!Theta || (T > 0 && (!times || !out)))))
+        return fail(h, RVL_EINVAL, "bad arguments");
+    if (!h->kids.empty()) {
+        const int rc = rvl_kepler_rv(h->kids[0], Theta, B, times, T, planet_mask, out, invalid, cap_hits);
+        return rc ? multi_fail(h, h->kids[0], rc) : RVL_OK;
+    }
+    if (!h->have_model) return fail(h, RVL_ESTATE, "set the model first");
+    if (B == 0) return RVL_OK;
+    DevGuard g(h->device);
+    int rc = ensure_io(h, B);
+    if (rc) return rc;
+    const size_t nT = (size_t)std::max(1, T), nout = (size_t)B * (size_t)T;
+    if (nT > h->cap_curve_t) {
+        cudaFree(h->d_curve_t);
+        h->d_curve_t = nullptr; h->cap_curve_t = 0;
+        CU(h, cudaMalloc(&h->d_curve_t, nT * sizeof(double)));
+        h->cap_curve_t = nT;
+    }
+    if (nout > h->cap_curve) {
+        cudaFree(h->d_curve);
+        h->d_curve = nullptr; h->cap_curve = 0;
+        CU(h, cudaMalloc(&h->d_curve, nout * sizeof(double)));
+        h->cap_curve = nout;
+    }
+    if (B > h->cap_curve_inv) {
+        cudaFree(h->d_curve_inv);
+        h->d_curve_inv = nullptr; h->cap_curve_inv = 0;
+        CU(h, cudaMalloc(&h->d_curve_inv, (size_t)B * sizeof(uint32_t)));
+        h->cap_curve_inv = B;
+    }
+    if (!h->d_curve_caps) CU(h, cudaMalloc(&h->d_curve_caps, sizeof(unsigned long long)));
+    cudaStream_t st = h->stream;
+    const size_t nb = (size_t)B * h->model.ndim * sizeof(double);
+    if (nb) CU(h, cudaMemcpyAsync(h->d_theta, Theta, nb, cudaMemcpyHostToDevice, st));
+    if (T > 0) CU(h, cudaMemcpyAsync(h->d_curve_t, times, (size_t)T * sizeof(double), cudaMemcpyHostToDevice, st));
+    CU(h, cudaMemsetAsync(h->d_curve_caps, 0, sizeof(unsigned long long), st));
+    rc = enqueue_kepler_rv(h, h->d_theta, B, h->d_curve_t, T, planet_mask, h->d_curve, h->d_curve_inv,
+                           h->d_curve_caps, st);
+    if (rc) return rc;
+    unsigned long long caps = 0;
+    if (nout) CU(h, cudaMemcpyAsync(out, h->d_curve, nout * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (invalid)
+        CU(h, cudaMemcpyAsync(invalid, h->d_curve_inv, (size_t)B * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CU(h, cudaMemcpyAsync(&caps, h->d_curve_caps, sizeof caps, cudaMemcpyDeviceToHost, st));
+    CU(h, cudaStreamSynchronize(st));
+    if (cap_hits) *cap_hits += caps;
+    return RVL_OK;
 }
 
 int rvl_counters(rvl_t *h, rvl_counters_t *out)

@@ -81,6 +81,95 @@ def _keys(tab):
     return list(tab.columns) if hasattr(tab, "columns") else list(tab.keys())
 
 
+# ---------------------------------------------------------------------- model curves: host logic
+# Output of one rvl_kepler_rv call is capped: larger requests are cut into row chunks.
+CURVE_CHUNK_BYTES = 256 << 20
+
+
+def planet_mask(nplanets, planets=None, exclude=None):
+    """Bit mask (bit p = planet p + 1) of the planets to sum: ``planets`` (a planet number 1..K or
+    an iterable of them; None = all) minus ``exclude`` (the same forms)."""
+    def numbers(sel, what):
+        if sel is None:
+            return []
+        sel = [sel] if np.ndim(sel) == 0 else list(sel)
+        out = []
+        for k in sel:
+            if int(k) != k or not 1 <= int(k) <= nplanets:
+                raise ValueError(f"{what}: {k!r} is not a planet number in 1..{nplanets}")
+            out.append(int(k))
+        return out
+    chosen = range(1, nplanets + 1) if planets is None else numbers(planets, "planets")
+    mask = 0
+    for k in chosen:
+        mask |= 1 << (k - 1)
+    for k in numbers(exclude, "exclude_planet"):
+        mask &= ~(1 << (k - 1))
+    return mask
+
+
+def curve_chunks(B, T, max_bytes=CURVE_CHUNK_BYTES):
+    """Row ranges [lo, hi) that cut a [B, T] float64 output into pieces of at most ``max_bytes``
+    (at least one row each)."""
+    rows = max(1, max_bytes // (8 * T)) if T > 0 else max(1, B)
+    return [(lo, min(B, lo + rows)) for lo in range(0, B, rows)]
+
+
+def planet_param_names(desc, k):
+    """(name, rvl_param) of every quantity that planet ``k`` (1-based) of a compiled
+    ``rvl_model_desc`` reads, in modelk's parametrisation (evidence/rvmodel/__init__.py:411-456)."""
+    pl = desc.planet[k - 1]
+    pre = f"planet{k}_"
+    e_names = {_abi.RVL_ECC_SECOS_SESIN: ("secos", "sesin"), _abi.RVL_ECC_ECOS_ESIN: ("ecos", "esin"),
+               _abi.RVL_ECC_DIRECT: ("ecc", "omega")}[pl.ecc_mode]
+    return [(pre + ("logk1" if pl.amp_is_log else "k1"), pl.amp),
+            (pre + ("logperiod" if pl.period_is_log else "period"), pl.period),
+            (pre + e_names[0], pl.e1), (pre + e_names[1], pl.e2),
+            (pre + ("ml0" if pl.phase_mode == _abi.RVL_PHASE_ML0 else "ma0"), pl.phase),
+            (pre + "epoch", pl.epoch)]
+
+
+def pardict_row(pardict, parnames, desc, mask):
+    """
+    theta row (sorted ``parnames`` order) for a reference-style ``pardict``, for the planets in
+    ``mask``.  Free names come from ``pardict``; a free name that none of those planets reads may be
+    missing and is filled with 0 (it cannot reach their velocities).  A missing free name that they
+    read raises KeyError, as the reference's lookup would.  The device model was compiled with the
+    fixed values, so a fixed name they read whose ``pardict`` value differs raises ValueError.
+    """
+    row = np.zeros(len(parnames), dtype=np.float64)
+    used = set()
+    for k in range(1, desc.n_planets + 1):
+        if not (mask >> (k - 1)) & 1:
+            continue
+        for name, par in planet_param_names(desc, k):
+            if par.slot >= 0:
+                used.add(par.slot)
+            elif name in pardict and float(pardict[name]) != par.value:
+                raise ValueError(f"{name} = {pardict[name]!r} differs from the model's fixed value "
+                                 f"{par.value!r}")
+    for i, name in enumerate(parnames):
+        if name in pardict:
+            row[i] = float(pardict[name])
+        elif i in used:
+            raise KeyError(name)
+    return row
+
+
+def host_drift(pardict, time):
+    """RVModel.drift (evidence/rvmodel/__init__.py:222-273) on the host, the reference's own
+    elementwise numpy arithmetic: lin*tt + quad*tt**2 + cub*tt**3 + quar*tt**4 with
+    tt = (time - tref)/365.25, tref = pardict['drift_tref'] if present, else time[0] of ``time``."""
+    time = np.asarray(time, dtype=np.float64)
+    lin = pardict.get("drift_lin", 0.0)
+    quad = pardict.get("drift_quad", 0.0)
+    cub = pardict.get("drift_cub", 0.0)
+    quar = pardict.get("drift_quar", 0.0)
+    tref = pardict["drift_tref"] if "drift_tref" in pardict else time[0]
+    tt = (time - tref) / 365.25
+    return lin * tt + quad * tt ** 2 + cub * tt ** 3 + quar * tt ** 4
+
+
 def _first_key(tab):
     return _keys(tab)[0]
 
@@ -318,6 +407,116 @@ class RVModel(BaseModel):
             self._h, c_void_p(U.data_ptr()), B, c_void_p(theta.data_ptr()),
             c_void_p(lnl.data_ptr()), c_void_p(stream)))
         return theta, lnl
+
+    # ------------------------------------------------------------------ model curves
+    def kepler_rv_batch(self, X, time, planets=None):
+        """
+        Keplerian velocity of every row of ``X`` (theta, sorted-parnames order) at ``time``: the sum
+        over ``planets`` (planet numbers 1..K; None = all) of modelk, in planet order
+        (evidence/rvmodel/__init__.py:343-463).  Returns ``(rv[B, T], ok[B])``; a row with an
+        invalid Keplerian among the summed planets is NaN with ``ok`` False.  Solves that stopped
+        at the Newton cap (which the reference drops silently) raise a RuntimeWarning.
+        """
+        X = self._as_batch(X, "X")
+        time = np.ascontiguousarray(time, dtype=np.float64).reshape(-1)
+        mask = planet_mask(self.nplanets, planets)
+        B, T = X.shape[0], time.shape[0]
+        rv = np.empty((B, T), dtype=np.float64)
+        inv = np.zeros(B, dtype=np.uint32)
+        caps = c_uint64(0)
+        for lo, hi in curve_chunks(B, T):
+            self._check(self._lib.rvl_kepler_rv(
+                self._h, X[lo:].ctypes.data, hi - lo, time.ctypes.data, T, mask,
+                rv[lo:].ctypes.data, inv[lo:].ctypes.data, byref(caps)))
+        if caps.value:
+            import warnings
+            warnings.warn(f"{caps.value} Kepler solves stopped at the Newton cap "
+                          f"(itmax = {self._desc.itmax}); their last iterate was used",
+                          RuntimeWarning, stacklevel=2)
+        return rv, (inv & np.uint32(mask)) == 0
+
+    def kepler_rv_device(self, theta, times, planets=None, out=None):
+        """
+        ``kepler_rv_batch`` for CUDA float64 tensors ``theta[B, ndim]`` and ``times[T]``, enqueued
+        on torch's current stream.  Returns ``(rv[B, T], ok[B])`` as CUDA tensors (no cap report).
+        """
+        import torch
+        for name, v in (("theta", theta), ("times", times)):
+            if not (v.is_cuda and v.dtype == torch.float64 and v.is_contiguous()):
+                raise ValueError(f"{name} must be a contiguous CUDA float64 tensor")
+        if theta.dim() != 2 or theta.shape[1] != self.ndim or times.dim() != 1:
+            raise ValueError(f"need theta of shape (B, {self.ndim}) and 1-D times")
+        mask = planet_mask(self.nplanets, planets)
+        B, T = theta.shape[0], times.shape[0]
+        if out is None:
+            out = torch.empty((B, T), dtype=torch.float64, device=theta.device)
+        elif not (out.is_cuda and out.dtype == torch.float64 and out.is_contiguous()
+                  and tuple(out.shape) == (B, T)):
+            raise ValueError(f"out must be a contiguous CUDA float64 tensor of shape ({B}, {T})")
+        inv = torch.zeros(B, dtype=torch.int32, device=theta.device)
+        stream = torch.cuda.current_stream(theta.device).cuda_stream
+        self._check(self._lib.rvl_kepler_rv_dev(
+            self._h, c_void_p(theta.data_ptr()), B, c_void_p(times.data_ptr()), T, mask,
+            c_void_p(out.data_ptr()), c_void_p(inv.data_ptr()), None, c_void_p(stream)))
+        return out, (inv & mask) == 0
+
+    def _curve(self, pardict, time, mask):
+        row = pardict_row(pardict, self.parnames, self._desc, mask)
+        time = np.asarray(time, dtype=np.float64).reshape(-1)
+        ks = [k for k in range(1, self.nplanets + 1) if (mask >> (k - 1)) & 1]
+        rv, ok = self.kepler_rv_batch(row[None], time, ks if ks else [])
+        return rv[0] if ok[0] else None
+
+    def modelk(self, pardict, time, planet):
+        """Velocity of planet ``planet`` (1..K) at ``time`` (evidence/rvmodel/__init__.py:388-463);
+        None for an invalid Keplerian (e > 1)."""
+        return self._curve(pardict, time, planet_mask(self.nplanets, planet))
+
+    def kep_rv(self, pardict, time, exclude_planet=None):
+        """Sum of the planets' velocities at ``time`` (evidence/rvmodel/__init__.py:343-385); None
+        if a summed planet is invalid.  ``exclude_planet``: a planet number, or an iterable of
+        them, left out of the sum (what a phase fold of one planet subtracts)."""
+        return self._curve(pardict, time, planet_mask(self.nplanets, exclude=exclude_planet))
+
+    def drift(self, pardict, time):
+        """evidence/rvmodel/__init__.py:222-273, on the host (see ``host_drift``)."""
+        return host_drift(pardict, time)
+
+    def residuals_batch(self, X):
+        """
+        Residuals and variances at the data epochs for every row of ``X``, composed in the
+        reference's order (evidence/rvmodel/__init__.py:183-215): rvm = offset[inst] + kep_rv
+        (device) + drift + sum of linear-parameter terms; res = vrad - rvm, var = svrad**2
+        (+ jitter**2).  Returns ``(res[B, N], var[B, N])``; rows with an invalid Keplerian are NaN.
+        """
+        X = self._as_batch(X, "X")
+        B = X.shape[0]
+        d = self._desc
+
+        def column(par):  # a model quantity for every row: a theta column or the fixed value
+            return X[:, par.slot] if par.slot >= 0 else np.full(B, par.value)
+        ids = self._inst_id
+        rvm = np.zeros((B, len(self.time)))
+        rvm += np.stack([column(d.offset[i]) for i in range(len(self.insts))], 1)[:, ids]
+        ok = np.ones(B, dtype=bool)
+        if self.nplanets > 0:
+            kep, ok = self.kepler_rv_batch(X, self.time)
+            rvm += kep
+        if self.drift_in_model:
+            coef = {nm: column(d.drift[j])[:, None]
+                    for j, nm in enumerate(("lin", "quad", "cub", "quar"))}
+            tt = (self.time - d.tref) / 365.25
+            rvm += (coef["lin"] * tt + coef["quad"] * tt ** 2 + coef["cub"] * tt ** 3
+                    + coef["quar"] * tt ** 4)
+        for j, name in enumerate(self.linpar_dict):
+            rvm += column(d.linpar[j])[:, None] * np.asarray(self.linpar_dict[name], dtype=np.float64)
+        res = self.vrad - rvm
+        var = np.broadcast_to(self.svrad ** 2, res.shape).copy()
+        if self.jitter_in_model:
+            var += np.stack([column(d.jitter[i]) for i in range(len(self.insts))], 1)[:, ids] ** 2
+        res[~ok] = np.nan
+        var[~ok] = np.nan
+        return res, var
 
     # ------------------------------------------------------------------ host helpers
     def linear_parameter(self, time, indicator, kernel=None, timescale=0.5, filter_type="lp"):

@@ -270,6 +270,27 @@ int rvl_wait_host_flags(const uint64_t *flags, int32_t n, uint64_t seq, int32_t 
 int rvl_trueanomaly(rvl_t *h, const double *M, int32_t n, double ecc, double *nu,
                     int32_t niterationmax, double tol);
 
+/* ---- model velocity curves: RVModel.kep_rv / modelk (evidence/rvmodel/__init__.py:343-463) ---- */
+/* Keplerian part of the model velocity for B theta rows at T caller times:
+ *   out[b][j] = sum over the planets p with bit p of planet_mask set, in planet order (kep_rv :383),
+ *               of modelk(theta_b, times[j], planet = p + 1)   (:388-463)
+ * planet_mask == 0 -> zeros; a bit at or above n_planets -> RVL_EINVAL.  invalid[b] (may be NULL):
+ * bit p set when planet p of row b is not a valid Keplerian (e > 1 in the secos/sesin or ecos/esin
+ * parametrisation, :425-439); a row with an invalid planet inside planet_mask is NaN.  cap_hits
+ * (may be NULL): incremented by the solves that stopped at itmax.  Needs rvl_set_model; Newton
+ * tol/itmax are the model's.  Times may be in any order and anywhere (|M| >= 1e5 takes the general
+ * Newton loop).  Each element is computed alone: a row's curve does not depend on the batch.  A
+ * multi-device handle runs the call on its first device (as rvl_trueanomaly does).  rvl_counters
+ * is not touched.  Synchronous. */
+int rvl_kepler_rv(rvl_t *h, const double *Theta, int64_t B, const double *times, int32_t T,
+                  uint32_t planet_mask, double *out, uint32_t *invalid, uint64_t *cap_hits);
+/* the same on device pointers (dCapHits: a device counter, may be NULL), asynchronous on stream;
+ * single-device handle; shares the handle's per-point scratch with the likelihood calls (stream
+ * order, as for every *_dev call) */
+int rvl_kepler_rv_dev(rvl_t *h, const double *dTheta, int64_t B, const double *dTimes, int32_t T,
+                      uint32_t planet_mask, double *dOut, uint32_t *dInvalid, uint64_t *dCapHits,
+                      void *stream);
+
 /* ---- observability / measurement ---------------------------------------- */
 int rvl_counters(rvl_t *h, rvl_counters_t *out);
 int rvl_reset_counters(rvl_t *h);
