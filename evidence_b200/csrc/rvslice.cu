@@ -15,7 +15,8 @@
 //                 their shrunken bracket and m more candidates (then: likelihood, slice_end again)
 //
 // One warp per walker, lanes over the dimensions (ndim <= 128).  Random numbers: Philox4x32-10
-// keyed by (seed, walker), counter = (move, draw) -- reproducible whatever the launch geometry.
+// keyed by the seed, counter = (move, draw, walker, 0) -- every (seed, move, draw, walker) has its
+// own stream, reproducible whatever k or the launch geometry.
 // Candidates outside the unit cube are clamped before evaluation and flagged, never accepted.
 #include <cuda_runtime.h>
 #include <math.h>
@@ -47,11 +48,12 @@ __device__ __forceinline__ U4 philox(U4 c, uint32_t k0, uint32_t k1)
     }
     return c;
 }
-// 53-bit uniform in (0, 1) from two words
+// uniform strictly inside (0, 1) from two words: 52 bits, ((v >> 1) + 0.5) 2^-52 is exact and lies
+// in [2^-53, 1 - 2^-53] ((2^53 - 1) + 0.5 would round to 2^53, i.e. exactly 1.0)
 __device__ __forceinline__ double u01(uint32_t a, uint32_t b)
 {
     const uint64_t v = ((uint64_t)a << 21) ^ (uint64_t)(b >> 11);  // 53 bits
-    return ((double)(v & ((1ull << 53) - 1)) + 0.5) * 0x1p-53;
+    return ((double)(v >> 1) + 0.5) * 0x1p-52;
 }
 
 struct SliceArgs {
@@ -83,6 +85,15 @@ struct SliceArgs {
 
 constexpr double kHiClamp = 1.0 - 0x1p-53;
 
+// the words of draw `tag` of walker w in this move.  The key is the seed alone and the walker is a
+// counter word: Philox is a bijection of the counter under a fixed key, so no two (seed, walker)
+// pairs share a stream (a key mixing seed and walker, e.g. seed ^ walker, would repeat across seeds)
+__device__ __forceinline__ U4 draw(const SliceArgs &a, uint32_t tag, int w)
+{
+    return philox(U4{a.move, tag, (uint32_t)w, 0u}, (uint32_t)a.seed,
+                  (uint32_t)(a.seed >> 32) + 0x51CEu);
+}
+
 __device__ __forceinline__ void write_candidate(const SliceArgs &a, double *cand, uint8_t *inside,
                                                 int w, int slot, int C, double t, const double *ui,
                                                 const double *di, int lane)
@@ -104,8 +115,7 @@ __device__ __forceinline__ void propose_shrink(const SliceArgs &a, int w, double
 {
     const int C = a.m;
     for (int j = 0; j < a.m; ++j) {
-        const U4 r = philox(U4{a.move, 0x53480000u + a.shrink_round * 64u + (uint32_t)j, 0u, 0u},
-                            (uint32_t)a.seed ^ (uint32_t)w, (uint32_t)(a.seed >> 32) + 0x51CEu);
+        const U4 r = draw(a, 0x53480000u + a.shrink_round * 64u + (uint32_t)j, w);
         const double t = lo + (hi - lo) * u01(r.x, r.y);
         if (lane == 0) a.tval[(size_t)w * a.m + j] = t;
         write_candidate(a, a.cand, a.inside, w, j, C, t, ui, di, lane);
@@ -123,8 +133,7 @@ __global__ void __launch_bounds__(128) slice_begin_kernel(const SliceArgs a)
     // z ~ N(0, I): Box-Muller on Philox words, two normals per counter
     double n2 = 0.0;
     for (int j = lane; j < a.d; j += 32) {
-        const U4 r = philox(U4{a.move, 0x44495200u + (uint32_t)(j >> 1), 0u, 0u},
-                            (uint32_t)a.seed ^ (uint32_t)w, (uint32_t)(a.seed >> 32) + 0x51CEu);
+        const U4 r = draw(a, 0x44495200u + (uint32_t)(j >> 1), w);
         const double rad = sqrt(-2.0 * log(u01(r.x, r.y))), ang = 6.283185307179586 * u01(r.z, r.w);
         const double v = (j & 1) ? rad * sin(ang) : rad * cos(ang);
         z[j] = v;
@@ -142,8 +151,7 @@ __global__ void __launch_bounds__(128) slice_begin_kernel(const SliceArgs a)
         di[j] = acc * inv;
     }
     __syncwarp();
-    const U4 r = philox(U4{a.move, 0x42524B00u, 0u, 0u}, (uint32_t)a.seed ^ (uint32_t)w,
-                        (uint32_t)(a.seed >> 32) + 0x51CEu);
+    const U4 r = draw(a, 0x42524B00u, w);
     const double r0 = u01(r.x, r.y);
     const double lo = -r0, hi = 1.0 - r0;
     if (lane == 0) { a.lo[w] = lo; a.hi[w] = hi; a.pending[w] = 1; }

@@ -363,7 +363,8 @@ void rvl_post_release(void);
  * rvl_transform_loglike_dev on `cand_out` (k * 2 n_out rows -> `ll_out`) after phase 0 and on
  * `cand` (k * m rows -> `cand_th`, `cand_ll`) after phases 1 and 2.  Candidates outside the unit cube are clamped for the evaluation and never accepted.
  * All pointers are device addresses (as 64-bit integers); random numbers are Philox4x32-10 keyed by
- * (seed, walker) with (move, shrink_round, draw) as the counter: reproducible for a seed.
+ * the seed with (move, shrink_round and draw, walker, 0) as the counter: every walker of every seed
+ * has its own streams, reproducible for a seed whatever k.
  * evidence_b200/sampler_dev.py drives it. */
 typedef struct {
     int32_t k, d, n_out, m;
