@@ -191,6 +191,34 @@ __device__ __forceinline__ int lds_u8(uint32_t addr)
     return (int)v;
 }
 
+// ---- the sin/cos table of rvl::sincos_tab (rvl_sintab.h) ---------------------------------------
+// In global memory as two arrays, the (sin, cos) hi parts and then the lo parts; every block that
+// runs the lean Newton loop copies both into its shared memory once, and the loop reads them
+// through SmemSinTab.  Two arrays rather than one of whole rows: a 16-byte load of rows with a
+// 16-byte stride spreads 32 random rows over twice the banks that a 32-byte stride would.
+__device__ const double2 g_sintab_hi[rvl::kSinTabN] = {RVL_SINTAB(RVL_SINTAB_HI_ROW)};
+__device__ const double2 g_sintab_lo[rvl::kSinTabN] = {RVL_SINTAB(RVL_SINTAB_LO_ROW)};
+constexpr unsigned kSinTabHiBytes = rvl::kSinTabN * sizeof(double2);
+constexpr unsigned kSinTabBytes = 2 * kSinTabHiBytes;
+static_assert(kSinTabBytes % 128 == 0, "the epoch columns behind the table stay 128-byte aligned");
+
+struct SmemSinTab {
+    uint32_t hi;  // shared-window address of the hi rows; the lo rows follow them
+    __device__ __forceinline__ rvl::TabRow operator()(int32_t j) const
+    {
+        // (not volatile: the table does not change once it is in shared memory, so the loads
+        // may be scheduled like arithmetic)
+        rvl::TabRow t;
+        // one address for both loads (left to itself the compiler shifts, masks and adds)
+        uint32_t a;
+        asm("mad.lo.u32 %0, %1, 16, %2;" : "=r"(a) : "r"(j), "r"(hi));
+        asm("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(t.sh), "=d"(t.ch) : "r"(a));
+        asm("ld.shared.v2.f64 {%0, %1}, [%2+16384];" : "=d"(t.sl), "=d"(t.cl) : "r"(a));
+        return t;
+    }
+};
+static_assert(kSinTabHiBytes == 16384, "SmemSinTab addresses the lo rows at +16384");
+
 // huge / non-finite arguments: CUDA libdevice (Payne-Hanek), out of line and returned by value
 __device__ __noinline__ double2 sincos_slow(double x)
 {
@@ -349,9 +377,9 @@ __device__ __forceinline__ void solve_planet_ref(const rvl::KTab &kt, const doub
 //     exit is then reached from the last pass alone and takes (sin E, cos E) from the registers
 //     that pass left them in (a join in front of the velocity formula cost 16 moves per 4 solves).
 template <int VARIANT, int U>
-__device__ __forceinline__ void solve_planet(const rvl::KTab &kt, const double (&t)[U], uint32_t pc, double tol,
-                                             int itmax, double (&rv)[U], int (&iters)[U],
-                                             int &caps, bool lean)
+__device__ __forceinline__ void solve_planet(const rvl::KTab &kt, SmemSinTab tab, const double (&t)[U],
+                                             uint32_t pc, double tol, int itmax, double (&rv)[U],
+                                             int (&iters)[U], int &caps, bool lean)
 {
     if (VARIANT != 0) {
         solve_planet_ref<VARIANT, U>(kt, t, pc, tol, itmax, rv, iters, caps);
@@ -371,7 +399,7 @@ __device__ __forceinline__ void solve_planet(const rvl::KTab &kt, const double (
         // pass 1 + step 1: E0 = M, every lane active (trueanomaly.c:19-29)
 #pragma unroll
         for (int u = 0; u < U; ++u) {
-            rvl::sincos_fast(kt, M[u], s[u], c[u]);
+            rvl::sincos_tab(kt, tab, M[u], s[u], c[u]);
             double En;
             rvl::newton_step(M[u], s[u], c[u], M[u], ec, En);
             d[u] = rvl::sub(En, M[u]);  // exact
@@ -401,7 +429,8 @@ __device__ __forceinline__ void solve_planet(const rvl::KTab &kt, const double (
                 if (wmax < kHiMid) {
 #pragma unroll
                     for (int u = 0; u < U; ++u) rvl::advance_mid(kt, d[u], s[u], c[u]);
-                } else {
+                } else {  // (a fresh sincos_tab here has fewer instructions, but measured slower:
+                          // its two table loads per solve cost more than the five FP64 saved)
 #pragma unroll
                     for (int u = 0; u < U; ++u) rvl::advance_medium(kt, d[u], s[u], c[u]);
                 }
@@ -409,7 +438,7 @@ __device__ __forceinline__ void solve_planet(const rvl::KTab &kt, const double (
                 // |E| can only leave the fast range after >= 3 Newton steps (|step| <= 100 |f|)
                 if (trip > 2 && any_big<U>(E)) { fallback = true; break; }
 #pragma unroll
-                for (int u = 0; u < U; ++u) rvl::sincos_fast(kt, E[u], s[u], c[u]);
+                for (int u = 0; u < U; ++u) rvl::sincos_tab(kt, tab, E[u], s[u], c[u]);
             }
             if (trip >= itmax) {  // the cap (trueanomaly.c:32-33): rare, finished on the spot so that
                                   // the common exit below is reached from the last pass alone and
@@ -579,8 +608,8 @@ struct ItemSums {
 #define RVL_ITEM_INLINE __forceinline__
 #endif
 template <int VARIANT, int U>
-__device__ RVL_ITEM_INLINE ItemSums item_epochs(const rvl::KTab &kt, const HotCtx *hc, uint32_t a_wc_in,
-                                                int c_lo, int c_hi, int lane)
+__device__ RVL_ITEM_INLINE ItemSums item_epochs(const rvl::KTab &kt, SmemSinTab tab, const HotCtx *hc,
+                                                uint32_t a_wc_in, int c_lo, int c_hi, int lane)
 {
 #if RVL_PIN_WC
     // the address of the warp's constants is needed once per planet and epoch group; left to
@@ -628,7 +657,7 @@ __device__ RVL_ITEM_INLINE ItemSums item_epochs(const rvl::KTab &kt, const HotCt
         for (int p = 0; p < K; ++p) {
             // each solve ADDS its planet's velocity to rvsum (kep_rv :383: the planets' sum, first
             // to last; 0 + v is v)
-            solve_planet<VARIANT, U>(kt, t, a_wc + (uint32_t)(p * kPlanetStride) * 8u, tol,
+            solve_planet<VARIANT, U>(kt, tab, t, a_wc + (uint32_t)(p * kPlanetStride) * 8u, tol,
                                      itmax, rvsum, it_l, cap_l, lean);
         }
         caps += cap_l;  // (padded / repeated lanes included: a cap hit is a cap hit)
@@ -715,8 +744,8 @@ template <int VARIANT, int U, int THREADS>
 __global__ void __launch_bounds__(THREADS, 1) rv_lnl_kernel(const KArgs a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    // [0,8) mbarrier, [16,128) HotCtx | [128, 128+sizeof(model)) model | epoch columns | inst ids |
-    // warp consts
+    // [0,8) mbarrier, [16,128) HotCtx | [128, 128+sizeof(model)) model | sin/cos table |
+    // epoch columns | inst ids | warp consts
     uint64_t *bar = reinterpret_cast<uint64_t *>(smem_raw);
     HotCtx *hc = reinterpret_cast<HotCtx *>(smem_raw + 16);
     static_assert(sizeof(HotCtx) <= 112, "HotCtx must fit in front of the model description");
@@ -731,10 +760,11 @@ __global__ void __launch_bounds__(THREADS, 1) rv_lnl_kernel(const KArgs a)
     const int nch0 = min(a.cpm, Ctot - c0);
     const int nch = U == 4 ? (nch0 + 3) / 4 * 4 : nch0;
     const int ne = nch * 32;
-    double *scol = reinterpret_cast<double *>(smem_raw + 128 + kModelBytes);
+    unsigned char *stab = smem_raw + 128 + kModelBytes;
+    double *scol = reinterpret_cast<double *>(stab + kSinTabBytes);
     uint8_t *sinst = reinterpret_cast<uint8_t *>(scol + (size_t)a.ncol * ne);
     double *wconst = reinterpret_cast<double *>(
-        smem_raw + 128 + kModelBytes + (((size_t)a.ncol * ne * 8 + ne + 127) / 128) * 128);
+        stab + kSinTabBytes + (((size_t)a.ncol * ne * 8 + ne + 127) / 128) * 128);
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     unsigned n_items = 0;
@@ -751,7 +781,9 @@ __global__ void __launch_bounds__(THREADS, 1) rv_lnl_kernel(const KArgs a)
     __syncthreads();
     if (tid == 0) {
         const unsigned col_bytes = (unsigned)ne * 8u;
-        mbar_expect_tx(bar, col_bytes * (unsigned)a.ncol + (unsigned)ne);
+        mbar_expect_tx(bar, col_bytes * (unsigned)a.ncol + (unsigned)ne + kSinTabBytes);
+        tma_load_1d(stab, g_sintab_hi, kSinTabHiBytes, bar);
+        tma_load_1d(stab + kSinTabHiBytes, g_sintab_lo, kSinTabBytes - kSinTabHiBytes, bar);
         for (int cidx = 0; cidx < a.ncol; ++cidx)
             tma_load_1d(scol + (size_t)cidx * ne, a.cols + (size_t)cidx * a.Npad + (size_t)c0 * 32,
                         col_bytes, bar);
@@ -801,11 +833,12 @@ __global__ void __launch_bounds__(THREADS, 1) rv_lnl_kernel(const KArgs a)
     }
     __syncthreads();
 
-    // the 17 constants of the sin/cos kernels, loaded once and kept (see rvl_math.h: KTab)
+    // the constants of the sin/cos kernels, loaded once and kept (see rvl_math.h: KTab)
 #ifndef RVL_PIN_KTAB
 #define RVL_PIN_KTAB 1
 #endif
     const rvl::KTab kt = RVL_PIN_KTAB ? rvl::load_ktab_pinned() : rvl::load_ktab();
+    const SmemSinTab tab{smem_u32(stab)};
     unsigned long long tot_iters = 0, tot_caps = 0, tot_invalid = 0;
     if (a.trace && lane == 0) {
         unsigned long long t;
@@ -886,7 +919,7 @@ __global__ void __launch_bounds__(THREADS, 1) rv_lnl_kernel(const KArgs a)
 
         // ---- the item's epochs: Kepler solves + Gaussian terms (out of line, see item_epochs) ----
         ItemSums sums{0.0, 1.0, 0, 0, 0, 1};
-        if (valid) sums = item_epochs<VARIANT, U>(kt, hc, a_wc, c_lo, c_hi, lane);
+        if (valid) sums = item_epochs<VARIANT, U>(kt, tab, hc, a_wc, c_lo, c_hi, lane);
         double chi = sums.chi, prod = sums.prod;
         int esum = sums.esum;
         const int iters = sums.iters, caps = sums.caps;
@@ -1260,9 +1293,19 @@ __global__ void __launch_bounds__(256, RVL_CURVE_MINB) kepler_rv_kernel(const Cu
 {
     static_assert(U == 2, "cap-hit accounting of the padding assumes two slots per lane");
     __shared__ __align__(16) double s_pc[8][RVL_MAX_PLANETS * kPlanetStride];
+    __shared__ __align__(16) unsigned char s_tab[kSinTabBytes];  // the likelihood kernel's table
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     double *wc = s_pc[warp];
     const uint32_t a_wc = smem_u32(wc);
+    {
+        const uint4 *hi = reinterpret_cast<const uint4 *>(g_sintab_hi);
+        const uint4 *lo = reinterpret_cast<const uint4 *>(g_sintab_lo);
+        uint4 *dst = reinterpret_cast<uint4 *>(s_tab);
+        constexpr int nhi = kSinTabHiBytes / 16, n = kSinTabBytes / 16;
+        for (int i = threadIdx.x; i < n; i += blockDim.x) dst[i] = i < nhi ? hi[i] : lo[i - nhi];
+        __syncthreads();
+    }
+    const SmemSinTab tab{smem_u32(s_tab)};
     const rvl::KTab kt = rvl::load_ktab_pinned();
     const int K = a.K, T = a.T, G = a.G;
     // the launch-wide conditions of the lean Newton loop (item_epochs)
@@ -1318,7 +1361,7 @@ __global__ void __launch_bounds__(256, RVL_CURVE_MINB) kepler_rv_kernel(const Cu
                     in_range = in_range &&
                                fabs(rvl::mean_anomaly(nmot, t[u], epoch, M0)) < 0.99 * rvl::kTrigFastMax;
                 const bool lean = lean_ok && __all_sync(kFull, in_range);
-                solve_planet<0, U>(kt, t, pc, a.tol, a.itmax, rv, it_l, cap_l, lean);
+                solve_planet<0, U>(kt, tab, t, pc, a.tol, a.itmax, rv, it_l, cap_l, lean);
             }
         }
         double *o = a.out + b * (long long)T;
@@ -1564,7 +1607,7 @@ struct Plan {
 
 size_t smem_need(int ncol, int ne, int W, int wstride)
 {
-    return 128 + kModelBytes + (((size_t)ncol * ne * 8 + ne + 127) / 128) * 128 +
+    return 128 + kModelBytes + kSinTabBytes + (((size_t)ncol * ne * 8 + ne + 127) / 128) * 128 +
            (size_t)W * wstride * 8;
 }
 
