@@ -125,6 +125,8 @@ SYMBOLS = {
     "rvl_order_last_error": (c_char_p, []),
     "rvl_post_release": (None, []),
     "rvl_slice_phase": (c_int32, [c_int32, POINTER(rvl_slice_args), c_void_p]),
+    "rvl_slice_phase_wrapped": (c_int32, [c_int32, POINTER(rvl_slice_args), POINTER(ctypes.c_uint32),
+                                          c_void_p]),
     "rvl_slice_last_error": (c_char_p, []),
     "rvl_plan_describe": (c_int32, [POINTER(c_int32), c_int64, POINTER(c_int64), c_int32]),
 }

@@ -18,11 +18,15 @@
 // keyed by the seed, counter = (move, draw, walker, 0) -- every (seed, move, draw, walker) has its
 // own stream, reproducible whatever k or the launch geometry.
 // Candidates outside the unit cube are clamped before evaluation and flagged, never accepted.
+// Circular coordinates (rvl_slice_phase_wrapped, the kWrap = true instantiations) are instead taken
+// modulo 1 -- the candidate stores p - floor(p), with 1 -> 0 -- and never flag a candidate: the
+// sampler then moves on the torus, whose uniform measure is the same as the cube's.
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
 
 #include <string>
+#include <type_traits>
 
 #include "../../include/rvlnl.h"
 
@@ -82,6 +86,13 @@ struct SliceArgs {
     const double *cand_th;   // [k][m][d]
     unsigned long long *stats;  // [0] walkers left pending by a slice_end, [1] accepted moves
 };
+// the arguments of the kWrap = true kernels: the mask by value after the fields of SliceArgs, which
+// keep their parameter offsets (and the kWrap = false kernels are exactly the unwrapped ones)
+struct SliceArgsWrap : SliceArgs {
+    uint32_t wrap[4];  // bit j & 31 of wrap[j >> 5]: coordinate j is circular
+};
+template <bool kWrap>
+using ArgsT = typename std::conditional<kWrap, SliceArgsWrap, SliceArgs>::type;
 
 constexpr double kHiClamp = 1.0 - 0x1p-53;
 
@@ -94,7 +105,8 @@ __device__ __forceinline__ U4 draw(const SliceArgs &a, uint32_t tag, int w)
                   (uint32_t)(a.seed >> 32) + 0x51CEu);
 }
 
-__device__ __forceinline__ void write_candidate(const SliceArgs &a, double *cand, uint8_t *inside,
+template <bool kWrap>
+__device__ __forceinline__ void write_candidate(const ArgsT<kWrap> &a, double *cand, uint8_t *inside,
                                                 int w, int slot, int C, double t, const double *ui,
                                                 const double *di, int lane)
 {
@@ -102,6 +114,18 @@ __device__ __forceinline__ void write_candidate(const SliceArgs &a, double *cand
     double *dst = cand + ((size_t)w * C + slot) * a.d;
     for (int j = lane; j < a.d; j += 32) {
         const double p = ui[j] + t * di[j];
+        if constexpr (kWrap) {
+            // constant word indices: the mask stays in the parameter bank (no local copy)
+            const uint32_t word = j < 32 ? a.wrap[0] : j < 64 ? a.wrap[1] : j < 96 ? a.wrap[2] : a.wrap[3];
+            if ((word >> (j & 31)) & 1u) {
+                // floor and the subtraction are exact; q rounds to 1.0 only for p in (-2^-54, 0),
+                // where 1 is the same point as 0
+                double q = p - floor(p);
+                if (q >= 1.0) q = 0.0;
+                dst[j] = q;
+                continue;
+            }
+        }
         in = in && (p >= 0.0) && (p < 1.0);
         dst[j] = fmin(fmax(p, 0.0), kHiClamp);
     }
@@ -110,7 +134,8 @@ __device__ __forceinline__ void write_candidate(const SliceArgs &a, double *cand
 }
 
 // the next m shrinkage candidates of walker w from bracket (lo, hi): sequential rule, speculated
-__device__ __forceinline__ void propose_shrink(const SliceArgs &a, int w, double lo, double hi,
+template <bool kWrap>
+__device__ __forceinline__ void propose_shrink(const ArgsT<kWrap> &a, int w, double lo, double hi,
                                                const double *ui, const double *di, int lane)
 {
     const int C = a.m;
@@ -118,13 +143,14 @@ __device__ __forceinline__ void propose_shrink(const SliceArgs &a, int w, double
         const U4 r = draw(a, 0x53480000u + a.shrink_round * 64u + (uint32_t)j, w);
         const double t = lo + (hi - lo) * u01(r.x, r.y);
         if (lane == 0) a.tval[(size_t)w * a.m + j] = t;
-        write_candidate(a, a.cand, a.inside, w, j, C, t, ui, di, lane);
+        write_candidate<kWrap>(a, a.cand, a.inside, w, j, C, t, ui, di, lane);
         if (t < 0.0) lo = t; else hi = t;
     }
     if (lane == 0) { a.lo2[w] = lo; a.hi2[w] = hi; }
 }
 
-__global__ void __launch_bounds__(128) slice_begin_kernel(const SliceArgs a)
+template <bool kWrap>
+__global__ void __launch_bounds__(128) slice_begin_kernel(const ArgsT<kWrap> a)
 {
     const int w = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (w >= a.k) return;
@@ -158,12 +184,13 @@ __global__ void __launch_bounds__(128) slice_begin_kernel(const SliceArgs a)
     const int C = 2 * a.n_out;
     const double *ui = a.u + (size_t)w * a.d;
     for (int j = 0; j < a.n_out; ++j) {
-        write_candidate(a, a.cand_o, a.inside_o, w, j, C, lo - (double)j, ui, di, lane);
-        write_candidate(a, a.cand_o, a.inside_o, w, a.n_out + j, C, hi + (double)j, ui, di, lane);
+        write_candidate<kWrap>(a, a.cand_o, a.inside_o, w, j, C, lo - (double)j, ui, di, lane);
+        write_candidate<kWrap>(a, a.cand_o, a.inside_o, w, a.n_out + j, C, hi + (double)j, ui, di, lane);
     }
 }
 
-__global__ void __launch_bounds__(128) slice_mid_kernel(const SliceArgs a)
+template <bool kWrap>
+__global__ void __launch_bounds__(128) slice_mid_kernel(const ArgsT<kWrap> a)
 {
     const int w = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (w >= a.k) return;
@@ -182,10 +209,11 @@ __global__ void __launch_bounds__(128) slice_mid_kernel(const SliceArgs a)
     const double lo = a.lo[w] - (double)run_lo, hi = a.hi[w] + (double)run_hi;
     __syncwarp();
     if (lane == 0) { a.lo[w] = lo; a.hi[w] = hi; }
-    propose_shrink(a, w, lo, hi, a.u + (size_t)w * a.d, a.dirn + (size_t)w * a.d, lane);
+    propose_shrink<kWrap>(a, w, lo, hi, a.u + (size_t)w * a.d, a.dirn + (size_t)w * a.d, lane);
 }
 
-__global__ void __launch_bounds__(128) slice_end_kernel(const SliceArgs a, int propose_more)
+template <bool kWrap>
+__global__ void __launch_bounds__(128) slice_end_kernel(const ArgsT<kWrap> a, int propose_more)
 {
     const int w = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (w >= a.k) return;
@@ -201,7 +229,8 @@ __global__ void __launch_bounds__(128) slice_end_kernel(const SliceArgs a, int p
         }
         if (first >= 0) {
             const size_t s = (size_t)w * C + first;
-            // the accepted point is the UNclamped candidate (it was inside the cube: identical)
+            // the accepted point is the UNclamped candidate (it was inside the cube: identical);
+            // a circular coordinate is the stored value, already taken modulo 1
             for (int j = lane; j < a.d; j += 32) {
                 ui[j] = a.cand[s * a.d + j];
                 a.theta[(size_t)w * a.d + j] = a.cand_th[s * a.d + j];
@@ -218,10 +247,10 @@ __global__ void __launch_bounds__(128) slice_end_kernel(const SliceArgs a, int p
     if (propose_more) {
         // still pending: m more candidates from the shrunken bracket; done: re-evaluate the current
         // point (keeps the launch shape fixed -- no compaction, no read-back)
-        if (pend) propose_shrink(a, w, a.lo2[w], a.hi2[w], ui, a.dirn + (size_t)w * a.d, lane);
+        if (pend) propose_shrink<kWrap>(a, w, a.lo2[w], a.hi2[w], ui, a.dirn + (size_t)w * a.d, lane);
         else
             for (int j = 0; j < a.m; ++j) {
-                write_candidate(a, a.cand, a.inside, w, j, C, 0.0, ui, a.dirn + (size_t)w * a.d, lane);
+                write_candidate<kWrap>(a, a.cand, a.inside, w, j, C, 0.0, ui, a.dirn + (size_t)w * a.d, lane);
                 if (lane == 0) a.inside[(size_t)w * C + j] = 0;
             }
     }
@@ -233,20 +262,25 @@ int sfail(const std::string &m)
     return RVL_EINVAL;
 }
 
-}  // namespace
-
-extern "C" {
-
-const char *rvl_slice_last_error(void) { return g_slice_error.c_str(); }
-
-/* One phase of a slice move (see the header).  p: 16 device pointers in the order of
- * rvl_slice_args; all launches go to `stream`. */
-int rvl_slice_phase(int32_t phase, const rvl_slice_args *s, void *stream)
+int slice_phase(int32_t phase, const rvl_slice_args *s, const uint32_t *wrap_bits, void *stream)
 {
     if (!s) return sfail("args is NULL");
     if (s->k <= 0 || s->d <= 0 || s->d > kMaxDim || s->n_out < 1 || s->m < 1 || s->m > 64)
         return sfail("bad sizes (k > 0, 0 < d <= 128, n_out >= 1, 1 <= m <= 64)");
-    SliceArgs a{};
+    SliceArgsWrap a{};
+    bool wrap = false;
+    if (wrap_bits) {
+        for (int i = 0; i < 4; ++i) {
+            // the bits at or above d of word i (word i holds coordinates 32 i .. 32 i + 31)
+            const int lo = s->d - 32 * i;
+            const uint32_t beyond = lo <= 0 ? 0xffffffffu : lo >= 32 ? 0u : ~((1u << lo) - 1u);
+            if (wrap_bits[i] & beyond)
+                return sfail("wrap_bits: bit " + std::to_string(32 * i + __builtin_ctz(wrap_bits[i] & beyond)) +
+                             " set, but d = " + std::to_string(s->d));
+            a.wrap[i] = wrap_bits[i];
+            wrap = wrap || wrap_bits[i] != 0u;
+        }
+    }
     a.k = s->k; a.d = s->d; a.n_out = s->n_out; a.m = s->m; a.seed = s->seed; a.move = s->move;
     a.shrink_round = s->shrink_round;
     a.lmin = (const double *)s->lmin; a.chol = (const double *)s->chol; a.u = (double *)s->u;
@@ -259,17 +293,45 @@ int rvl_slice_phase(int32_t phase, const rvl_slice_args *s, void *stream)
     const int wpb = 4;
     const unsigned grid = (unsigned)((s->k + wpb - 1) / wpb);
     cudaStream_t st = (cudaStream_t)stream;
-    if (phase == 0) slice_begin_kernel<<<grid, wpb * 32, 0, st>>>(a);
-    else if (phase == 1) slice_mid_kernel<<<grid, wpb * 32, 0, st>>>(a);
-    else if (phase == 2) slice_end_kernel<<<grid, wpb * 32, 0, st>>>(a, 1);
-    else if (phase == 3) slice_end_kernel<<<grid, wpb * 32, 0, st>>>(a, 0);
-    else return sfail("phase must be 0 (begin), 1 (mid), 2 (end + more candidates) or 3 (end)");
+    if (phase < 0 || phase > 3)
+        return sfail("phase must be 0 (begin), 1 (mid), 2 (end + more candidates) or 3 (end)");
+    if (wrap) {
+        if (phase == 0) slice_begin_kernel<true><<<grid, wpb * 32, 0, st>>>(a);
+        else if (phase == 1) slice_mid_kernel<true><<<grid, wpb * 32, 0, st>>>(a);
+        else slice_end_kernel<true><<<grid, wpb * 32, 0, st>>>(a, phase == 2 ? 1 : 0);
+    } else {
+        const SliceArgs &b = a;
+        if (phase == 0) slice_begin_kernel<false><<<grid, wpb * 32, 0, st>>>(b);
+        else if (phase == 1) slice_mid_kernel<false><<<grid, wpb * 32, 0, st>>>(b);
+        else slice_end_kernel<false><<<grid, wpb * 32, 0, st>>>(b, phase == 2 ? 1 : 0);
+    }
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) {
         g_slice_error = cudaGetErrorString(e);
         return RVL_ECUDA;
     }
     return RVL_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+const char *rvl_slice_last_error(void) { return g_slice_error.c_str(); }
+
+/* One phase of a slice move (see the header).  p: 16 device pointers in the order of
+ * rvl_slice_args; all launches go to `stream`. */
+int rvl_slice_phase(int32_t phase, const rvl_slice_args *s, void *stream)
+{
+    return slice_phase(phase, s, nullptr, stream);
+}
+
+/* The same with circular coordinates: bit j & 31 of wrap_bits[j >> 5] set = coordinate j is taken
+ * modulo 1 (see the header).  NULL or no bit set: exactly the launches of rvl_slice_phase. */
+int rvl_slice_phase_wrapped(int32_t phase, const rvl_slice_args *s, const uint32_t wrap_bits[4],
+                            void *stream)
+{
+    return slice_phase(phase, s, wrap_bits, stream);
 }
 
 }  // extern "C"

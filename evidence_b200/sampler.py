@@ -24,6 +24,14 @@ points (MultiNest with one ellipsoid / nestle's 'single' bound); candidates are 
 of ``ndraw`` -- the large batches the device path is built for -- and consumed in order.  Efficient
 for unimodal problems only.
 
+Circular coordinates (``wrapped``, UltraNest's ``wrapped_params``; opt-in): the slice samplers take
+a wrapped coordinate of every candidate modulo 1 instead of rejecting it outside [0, 1), so the
+walkers move on the torus (``wrap_unit``), and whiten with the covariance of the live points
+re-centred on their circular mean in those coordinates (``recentre``).  Nested sampling needs
+points uniform in the cube under L > L*; the torus has the same uniform measure, so this is valid
+for any coordinate and helps where lnL is periodic (an argument of periastron whose posterior
+straddles 0 = 2 pi is then one mode, not two on opposite faces of the cube).
+
 ln Z uncertainty: the larger of Skilling's estimate sqrt(H / nlive) and a bootstrap over the run's
 threads (``lineage_bootstrap``, the estimate UltraNest's ``num_bootstraps`` makes); likelihood
 plateaus (tied values, e.g. the model's -1e30) are retired as a whole (``retire_groups``).
@@ -259,7 +267,39 @@ def lineage_bootstrap(birth, death, root, n_roots, rng, num=30):
 # ------------------------------------------------------------------------------------------
 # slice-sampling replacement (default)
 # ------------------------------------------------------------------------------------------
-def _whitening(u):
+def wrap_mask(wrapped, ndim):
+    """The circular coordinates as a bool array [ndim] (all False for None)."""
+    if wrapped is None:
+        return np.zeros(ndim, dtype=bool)
+    w = np.asarray(wrapped, dtype=bool).reshape(-1)
+    if w.shape != (ndim,):
+        raise ValueError(f"wrapped: {len(w)} entries for {ndim} dimensions")
+    return w
+
+
+def wrap_unit(p):
+    """p modulo 1: p - floor(p) (exact), and 0 where that rounds to 1.0 -- only for p in
+    (-2^-54, 0), where 1 is the same point as 0.  The rule of rvl_slice_phase_wrapped."""
+    q = p - np.floor(p)
+    return np.where(q >= 1.0, 0.0, q)
+
+
+def recentre(u, wrapped):
+    """u[n, d] with every circular coordinate j moved to frac(u_j - mu_j + 1/2), mu_j the circular
+    mean atan2(mean sin 2 pi u_j, mean cos 2 pi u_j) / 2 pi: a mode that straddles the seam then
+    lies in the middle of [0, 1), and its covariance does not depend on where it sits."""
+    ang = 2.0 * np.pi * u[:, wrapped]
+    mu = np.arctan2(np.sin(ang).mean(axis=0), np.cos(ang).mean(axis=0)) / (2.0 * np.pi)
+    v = u.copy()
+    v[:, wrapped] = wrap_unit(u[:, wrapped] - mu + 0.5)
+    return v
+
+
+def _whitening(u, wrapped=None):
+    """Lower Cholesky factor of the covariance of the live points u[n, d]; circular coordinates
+    (``wrapped``, a bool mask with at least one True) about their circular mean."""
+    if wrapped is not None:
+        u = recentre(u, wrapped)
     d = u.shape[1]
     cov = np.cov(u.T).reshape(d, d) + np.eye(d) * 1e-18
     try:
@@ -269,14 +309,16 @@ def _whitening(u):
 
 
 def _slice_moves(rng, loglike, transform, u, lmin, chol, nsteps, max_expand=16, max_shrink=64,
-                 fused=None, speculate=None):
+                 fused=None, speculate=None, wrapped=None):
     """Advance k walkers u[k, d] by nsteps slice moves under L > lmin; all evaluations batched.
     ``fused(u) -> (theta, lnL)``, when given, replaces the transform + loglike pair of every
     evaluation by one call (one device round trip instead of two).  ``speculate`` = m: every call
     evaluates the next m stepping-out positions of both sides, and then the next m shrinkage
     candidates, of every walker at once.  The chain is EXACTLY the sequential one (m = 1) -- the
     extra evaluations are discarded -- but it needs ~3x fewer, larger device calls, which is
-    what a latency-bound accelerator wants.  None: chosen from the number of walkers."""
+    what a latency-bound accelerator wants.  None: chosen from the number of walkers.  ``wrapped``
+    (bool mask with at least one True, or None): those coordinates of every candidate are taken
+    modulo 1 before the cube test, and an accepted candidate keeps the wrapped value."""
     k, d = u.shape
     theta = transform(u)
     lcur = np.full(k, np.nan)
@@ -323,6 +365,8 @@ def _slice_moves(rng, loglike, transform, u, lmin, chol, nsteps, max_expand=16, 
                                    grow_hi[:, None] & (done_hi[:, None] + steps[None, :] < max_expand)],
                                   axis=1)
             pts = u[:, None, :] + edges[:, :, None] * dirn[:, None, :]
+            if wrapped is not None:
+                pts[..., wrapped] = wrap_unit(pts[..., wrapped])
             l_e, _ = evaluate(pts.reshape(-1, d), mask.reshape(-1))
             above = (l_e.reshape(k, 2 * m) > lmin) & mask
             run_lo = np.cumprod(above[:, :m], axis=1).sum(axis=1)              # leading successes
@@ -350,6 +394,8 @@ def _slice_moves(rng, loglike, transform, u, lmin, chol, nsteps, max_expand=16, 
                 lo_s = np.where(t < 0, t, lo_s)
                 hi_s = np.where(t >= 0, t, hi_s)
             cand = u[:, None, :] + T[:, :, None] * dirn[:, None, :]            # [k, mm, d]
+            if wrapped is not None:
+                cand[..., wrapped] = wrap_unit(cand[..., wrapped])
             l_c, th_c = evaluate(cand.reshape(-1, d), np.repeat(pending, mm))
             l_c = l_c.reshape(k, mm)
             acc = l_c > lmin
@@ -371,18 +417,29 @@ def _slice_moves(rng, loglike, transform, u, lmin, chol, nsteps, max_expand=16, 
 
 def nested_sample(loglike, transform, ndim, nlive=400, ndraw=4096, dlogz=0.5, frac_remain=0.01,
                   seed=0, nsteps=None, batch_fraction=0.2, method="slice", max_calls=500_000_000,
-                  verbose=False, fused=None, speculate=None, num_bootstraps=30, **kw):
+                  verbose=False, fused=None, speculate=None, num_bootstraps=30, wrapped=None, **kw):
     """
     Seeded vectorised nested sampling; see the module docstring.  ``loglike(theta[n, ndim])`` and
     ``transform(u[n, ndim])`` follow UltraNest's ``vectorized=True`` convention.  Returns a
     ``NestedResult`` (logz, logzerr, ncall, niter, samples, ...).  ``fused(u[n, ndim]) ->
     (theta[n, ndim], lnL[n])`` (method='slice'): the device's fused u -> theta -> lnL call; it must
     return what ``transform`` followed by ``loglike`` returns, and then the run is identical.
+    ``wrapped`` (bool per dimension, UltraNest's ``wrapped_params``): circular coordinates of the
+    slice method (module docstring); None or no True leaves the run exactly as without it.  The
+    result's ``wrapped`` holds the mask.
     """
+    wmask = wrap_mask(wrapped, ndim)
     if method == "ellipsoid":
-        return nested_sample_ellipsoid(loglike, transform, ndim, nlive=nlive, ndraw=ndraw,
-                                       dlogz=dlogz, frac_remain=frac_remain, seed=seed,
-                                       max_calls=max_calls, verbose=verbose, **kw)
+        if wmask.any():
+            # an ellipsoid longer than 1 along a circular axis covers some points twice: its
+            # proposal would not be uniform on the torus
+            raise ValueError("method='ellipsoid' does not support wrapped (circular) coordinates")
+        res = nested_sample_ellipsoid(loglike, transform, ndim, nlive=nlive, ndraw=ndraw,
+                                      dlogz=dlogz, frac_remain=frac_remain, seed=seed,
+                                      max_calls=max_calls, verbose=verbose, **kw)
+        res["wrapped"] = wmask
+        return res
+    wrap = wmask if wmask.any() else None
     rng = np.random.default_rng(seed)
     nsteps = nsteps or max(4, 3 * ndim)  # the reference's default (evidence/ultranest/__init__.py:335)
     k = max(1, min(int(batch_fraction * nlive), nlive - 2, ndraw))
@@ -426,11 +483,11 @@ def nested_sample(loglike, transform, ndim, nlive=400, ndraw=4096, dlogz=0.5, fr
         logx += float(np.sum(dlogx))
         lmin = l_live[worst[-1]]
         keep = order[kk:]
-        chol = _whitening(u_live[keep])
+        chol = _whitening(u_live[keep], wrap)
         starts = keep[rng.integers(0, len(keep), kk)]
         u_new, th_new, l_new, nc = _slice_moves(rng, loglike, transform, u_live[starts].copy(),
                                                 lmin, chol, nsteps, fused=fused,
-                                                speculate=speculate)
+                                                speculate=speculate, wrapped=wrap)
         ncall += nc
         stuck = ~np.isfinite(l_new)  # a walker that never moved is a copy of its start point
         l_new = np.where(stuck, l_live[starts], l_new)
@@ -473,4 +530,4 @@ def nested_sample(loglike, transform, ndim, nlive=400, ndraw=4096, dlogz=0.5, fr
                         logzerr_skilling=skilling, logzerr_bootstrap=bs_std,
                         ncall=int(ncall), niter=int(niter), information=float(h_info),
                         samples=theta[idx], weighted_samples=theta, weights=weights,
-                        logl=dead_logl, nlive=nlive, seed=seed, method="slice")
+                        logl=dead_logl, nlive=nlive, seed=seed, method="slice", wrapped=wmask)

@@ -17,7 +17,9 @@ m stepping-out positions and shrinkage candidates of every walker evaluated spec
 launch (see ``sampler._slice_moves``).  Differences from the numpy sampler: the random numbers come
 from torch's generator (so the two are statistically, not bit-wise, equivalent), and candidates
 outside the unit cube are clamped before they are evaluated and rejected afterwards (no compaction
-of the batch, hence no synchronisation to learn its size).
+of the batch, hence no synchronisation to learn its size).  Circular coordinates (``wrapped``) follow
+the rule of ``sampler``: taken modulo 1 in every candidate (``rvl_slice_phase_wrapped`` in the
+kernels), whitened about their circular mean.
 
 There is no CPU fallback in the product: ``fused`` must be a device callable.  (The function itself
 is device-agnostic torch code, which is how the CPU tests drive it with an analytic likelihood.)
@@ -26,10 +28,22 @@ import math
 
 import numpy as np
 
-from .sampler import NestedResult, lineage_bootstrap, retire_groups
+from .sampler import NestedResult, lineage_bootstrap, retire_groups, wrap_mask
 
 
-def _whitening(torch, u):
+def _wrap_unit(torch, p):
+    """p modulo 1 with 1 -> 0 (``sampler.wrap_unit``)."""
+    q = p - torch.floor(p)
+    return torch.where(q >= 1.0, torch.zeros_like(q), q)
+
+
+def _whitening(torch, u, wrapped=None):
+    """Lower Cholesky factor of the covariance of u[n, d]; ``wrapped`` (bool tensor [d] with at least
+    one True, or None): those coordinates about their circular mean (``sampler.recentre``)."""
+    if wrapped is not None:
+        ang = 2.0 * math.pi * u
+        mu = torch.atan2(torch.sin(ang).mean(0), torch.cos(ang).mean(0)) / (2.0 * math.pi)
+        u = torch.where(wrapped, _wrap_unit(torch, u - mu + 0.5), u)
     d = u.shape[1]
     cov = torch.cov(u.T).reshape(d, d) + torch.eye(d, dtype=u.dtype, device=u.device) * 1e-18
     L, info = torch.linalg.cholesky_ex(cov)
@@ -38,9 +52,10 @@ def _whitening(torch, u):
 
 
 def _slice_moves(torch, gen, fused, u, theta, lmin, chol, nsteps, m, max_expand, max_shrink,
-                 m_out=None):
+                 m_out=None, wrapped=None):
     """k walkers, nsteps slice moves each, everything on u.device.  Returns (u, theta, lnL, ncall);
-    lnL is NaN for a walker that never moved."""
+    lnL is NaN for a walker that never moved.  ``wrapped`` (bool tensor [d] or None): those
+    coordinates of every candidate are taken modulo 1 before the cube test and kept so."""
     k, d = u.shape
     dev, f64 = u.device, u.dtype
     lcur = torch.full((k,), float("nan"), dtype=f64, device=dev)
@@ -53,6 +68,9 @@ def _slice_moves(torch, gen, fused, u, theta, lmin, chol, nsteps, m, max_expand,
     isteps = torch.arange(mo, device=dev)
     hi_clamp = 1.0 - 2.0 ** -53
     ncall = 0
+
+    def fold(points):
+        return points if wrapped is None else torch.where(wrapped, _wrap_unit(torch, points), points)
 
     def evaluate(points):
         """lnL (and theta) of points[k, n, d]; -inf outside the unit cube."""
@@ -80,7 +98,7 @@ def _slice_moves(torch, gen, fused, u, theta, lmin, chol, nsteps, m, max_expand,
             edges = torch.cat([lo[:, None] - steps[None, :], hi[:, None] + steps[None, :]], dim=1)
             mask = torch.cat([grow_lo[:, None] & (done_lo[:, None] + isteps[None, :] < max_expand),
                               grow_hi[:, None] & (done_hi[:, None] + isteps[None, :] < max_expand)], dim=1)
-            ll, _ = evaluate(u[:, None, :] + edges[:, :, None] * dirn[:, None, :])
+            ll, _ = evaluate(fold(u[:, None, :] + edges[:, :, None] * dirn[:, None, :]))
             above = (ll > lmin) & mask
             run_lo = torch.cumprod(above[:, :mo].to(torch.long), dim=1).sum(dim=1)
             run_hi = torch.cumprod(above[:, mo:].to(torch.long), dim=1).sum(dim=1)
@@ -108,7 +126,7 @@ def _slice_moves(torch, gen, fused, u, theta, lmin, chol, nsteps, m, max_expand,
                 lo_s = torch.where(t < 0, t, lo_s)
                 hi_s = torch.where(t >= 0, t, hi_s)
             T = torch.stack(ts, dim=1)
-            cand = u[:, None, :] + T[:, :, None] * dirn[:, None, :]
+            cand = fold(u[:, None, :] + T[:, :, None] * dirn[:, None, :])
             ll, th = evaluate(cand)
             acc = (ll > lmin) & pending[:, None]
             hit = acc.any(dim=1)
@@ -132,10 +150,11 @@ class _NativeSlice:
     read back.  Stepping out evaluates all ``n_out`` positions of both sides at once; shrinkage runs
     ``rounds`` launches of ``m`` speculated candidates per walker (a walker whose bracket is not
     resolved after rounds * m candidates keeps its position -- counted in ``unresolved``; with the
-    defaults, 24 candidates, that is a few 1e-3 of the moves on the RV posteriors).
+    defaults, 24 candidates, that is a few 1e-3 of the moves on the RV posteriors).  ``wrap`` (bool
+    per dimension, or None): circular coordinates, through ``rvl_slice_phase_wrapped``.
     """
 
-    def __init__(self, torch, k, d, dev, seed, n_out=8, m=8, rounds=3):
+    def __init__(self, torch, k, d, dev, seed, n_out=8, m=8, rounds=3, wrap=None):
         import ctypes
         from . import _abi
         self.torch, self.k, self.d, self.n_out, self.m, self.rounds = torch, k, d, n_out, m, rounds
@@ -159,11 +178,19 @@ class _NativeSlice:
                         ("cand_th", self.th), ("stats", self.stats)):
             setattr(self.args, name, t.data_ptr())
         self._byref = ctypes.byref(self.args)
+        self.wrap_bits = None
+        if wrap is not None and np.any(wrap):
+            self.wrap_bits = (ctypes.c_uint32 * 4)()
+            for j in np.flatnonzero(np.asarray(wrap, dtype=bool)):
+                self.wrap_bits[j >> 5] |= 1 << (int(j) & 31)
         self.move = 0
 
     def _phase(self, ph):
         stream = self.torch.cuda.current_stream().cuda_stream
-        rc = self.lib.rvl_slice_phase(ph, self._byref, stream)
+        if self.wrap_bits is None:
+            rc = self.lib.rvl_slice_phase(ph, self._byref, stream)
+        else:
+            rc = self.lib.rvl_slice_phase_wrapped(ph, self._byref, self.wrap_bits, stream)
         if rc != 0:
             raise RuntimeError("rvl_slice_phase: " + self.lib.rvl_slice_last_error().decode())
 
@@ -210,7 +237,7 @@ class _NativeSlice:
 def nested_sample_device(fused, ndim, nlive=400, dlogz=0.5, frac_remain=0.01, seed=0, nsteps=None,
                          batch_fraction=0.2, speculate=None, device="cuda", max_expand=16,
                          max_shrink=64, max_calls=2_000_000_000, verbose=False, num_bootstraps=30,
-                         native=None, native_m=8, native_rounds=3, native_out=8):
+                         native=None, native_m=8, native_rounds=3, native_out=8, wrapped=None):
     """
     Nested sampling with every array on ``device``.  ``fused(U[n, ndim]) -> (theta[n, ndim],
     lnL[n])`` maps unit-cube points to parameters and log-likelihoods on that device
@@ -222,6 +249,9 @@ def nested_sample_device(fused, ndim, nlive=400, dlogz=0.5, frac_remain=0.01, se
     ``native_out`` stepping-out positions per side, ``native_rounds`` x ``native_m`` shrinkage
     candidates per walker and move, all speculated.  The torch formulation below it is the same
     sampler for CPU tensors (tests) and the statistical cross-check of the kernels.
+
+    ``wrapped`` (bool per dimension, UltraNest's ``wrapped_params``): circular coordinates, as in
+    ``sampler.nested_sample``; None or no True leaves the run exactly as without it.
     """
     import torch
     dev = torch.device(device)
@@ -230,6 +260,8 @@ def nested_sample_device(fused, ndim, nlive=400, dlogz=0.5, frac_remain=0.01, se
     if native is None:
         native = dev.type == "cuda"
     nsteps = nsteps or max(4, 3 * ndim)  # the reference's default (evidence/ultranest/__init__.py:335)
+    wmask = wrap_mask(wrapped, ndim)
+    wrap = torch.as_tensor(wmask, device=dev) if wmask.any() else None
     k = max(1, min(int(batch_fraction * nlive), nlive - 2))
     m = max(1, min(6, 512 // k)) if speculate is None else max(1, int(speculate))
     m_out = max(m, min(max_expand, 4096 // (2 * k)))  # a likelihood launch costs the same up to ~4096 points
@@ -272,12 +304,12 @@ def nested_sample_device(fused, ndim, nlive=400, dlogz=0.5, frac_remain=0.01, se
         logx -= dx
         niter += kk
         lmin = l_sorted[kk - 1]
-        chol = _whitening(torch, u_live[keep])
+        chol = _whitening(torch, u_live[keep], wrap)
         starts = keep[torch.randint(0, len(keep), (kk,), generator=gen, device=dev)]
         if native:
             if kk not in natives:
                 natives[kk] = _NativeSlice(torch, kk, ndim, dev, seed, n_out=native_out, m=native_m,
-                                           rounds=native_rounds)
+                                           rounds=native_rounds, wrap=wmask)
             natives[kk].move = move_no
             u_new, th_new = u_live[starts].clone(), th_live[starts].clone()
             l_new = torch.full((kk,), float("nan"), dtype=f64, device=dev)
@@ -286,7 +318,7 @@ def nested_sample_device(fused, ndim, nlive=400, dlogz=0.5, frac_remain=0.01, se
         else:
             u_new, th_new, l_new, nc = _slice_moves(torch, gen, fused, u_live[starts].clone(),
                                                     th_live[starts].clone(), lmin, chol, nsteps, m,
-                                                    max_expand, max_shrink, m_out=m_out)
+                                                    max_expand, max_shrink, m_out=m_out, wrapped=wrap)
         ncall += nc
         stuck = ~torch.isfinite(l_new)  # a walker that never moved is a copy of its start point
         l_new = torch.where(stuck, l_live[starts], l_new)
@@ -334,4 +366,5 @@ def nested_sample_device(fused, ndim, nlive=400, dlogz=0.5, frac_remain=0.01, se
                         weights=weights.cpu().numpy(), logl=logl.cpu().numpy(), nlive=nlive,
                         seed=seed, method="slice-device" + ("-native" if native else ""),
                         unresolved_moves=int(sum(int(n.stats[0]) for n in natives.values())),
-                        accepted_moves=int(sum(int(n.stats[1]) for n in natives.values())))
+                        accepted_moves=int(sum(int(n.stats[1]) for n in natives.values())),
+                        wrapped=wmask)

@@ -13,6 +13,8 @@ Extra ``ultrasettings`` keys (the "config switch"):
     'vectorized' (True), 'ndraw_min' (4096), 'ndraw_max' (65536), 'seed' (None),
     'stepsampler' ('region-slice' like the reference | 'population-slice' | 'none'),
     'sampler' ('auto' | 'ultranest' | 'builtin'), 'builtin_method' ('slice' | 'slice-device' | 'ellipsoid'),
+    'builtin_wrap' (False: the built-in slice samplers take the wrapped parameters -- the ones UltraNest
+    gets as ``wrapped_params`` -- as circular coordinates; 'ellipsoid' rejects it),
     'postprocess' (False), 'plot' (False)
 
 UltraNest is a third-party package that is not part of the reference repository (SURVEY.md 8c).
@@ -132,6 +134,8 @@ def run(model, rundict, priordict, ultrasettings=None):
         os.makedirs(settings["log_dir"], exist_ok=True)
         # the device model evaluates u -> theta -> lnL in one call (rvl_transform_loglike)
         fused = getattr(model, "transform_loglike_batch", None) if hasattr(model, "set_priors") else None
+        # the circular parameters UltraNest gets, only when asked for
+        builtin_wrapped = wrapped if settings["builtin_wrap"] else None
         if settings["builtin_method"] == "slice-device":
             # the whole run on the likelihood's device (evidence_b200.sampler_dev)
             from .sampler_dev import nested_sample_device
@@ -141,12 +145,12 @@ def run(model, rundict, priordict, ultrasettings=None):
                                        nlive=settings["nlive"], dlogz=settings["dlogz"],
                                        frac_remain=settings["frac_remain"], nsteps=settings["nsteps"],
                                        seed=0 if settings["seed"] is None else settings["seed"],
-                                       device=_torch_device(model))
+                                       device=_torch_device(model), wrapped=builtin_wrapped)
         else:
             res = nested_sample(loglike, prior, ndim, nlive=settings["nlive"], fused=fused,
                                 ndraw=settings["ndraw_min"], dlogz=settings["dlogz"],
                                 frac_remain=settings["frac_remain"], nsteps=settings["nsteps"],
-                                method=settings["builtin_method"],
+                                method=settings["builtin_method"], wrapped=builtin_wrapped,
                                 seed=0 if settings["seed"] is None else settings["seed"])
         logz, logzerr, ncall, samples = res.logz, res.logzerr, res.ncall, res.samples
         # the reference's post-processing knows 'PolyChord' and 'UltraNest' only and, for the latter,
@@ -154,6 +158,8 @@ def run(model, rundict, priordict, ultrasettings=None):
         # file, and the implementation named beside it
         name = "UltraNest"
         impl = f"evidence_b200.sampler ({settings['builtin_method']}); ultranest not used"
+        if builtin_wrapped is not None:
+            impl += "; wrapped: " + (", ".join(p for p, w in zip(parnames, wrapped) if w) or "none")
         write_weighted_post(settings["log_dir"], parnames, res)
     tf = time.process_time()
     t_wall = time.perf_counter() - t_wall
@@ -232,6 +238,7 @@ def set_ultrasettings(rundict, ultrasettings, ndim, nderived, isodate, parnames)
                 # the device-path switch
                 "vectorized": True, "ndraw_min": 4096, "ndraw_max": 65536, "seed": None,
                 "stepsampler": "region-slice", "sampler": "auto", "builtin_method": "slice",
+                "builtin_wrap": False,
                 "postprocess": False, "plot": False}
     if ultrasettings is not None:
         if type(ultrasettings) is not dict:

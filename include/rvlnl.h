@@ -389,6 +389,18 @@ typedef struct {
     uint64_t stats;   /* uint64_t*      [2]        += walkers left unresolved, += accepted moves */
 } rvl_slice_args;
 int rvl_slice_phase(int32_t phase, const rvl_slice_args *args, void *stream);
+/* rvl_slice_phase with circular coordinates: bit j & 31 of wrap_bits[j >> 5] set marks coordinate j
+ * as circular (UltraNest's wrapped_params; the reference wraps names containing "omega" or "ml0",
+ * evidence/ultranest/__init__.py:159-162).  A candidate's circular coordinate p = u + t dirn is
+ * stored as q = p - floor(p), with q = 0 where that rounds to 1 (only for a tiny negative p), and
+ * never marks the candidate as outside the cube; an accepted point is that stored value, so u stays
+ * in [0, 1).  The other coordinates, directions, brackets, random streams and acceptance are those
+ * of rvl_slice_phase.  The walkers then move on the torus, whose uniform measure is the cube's: the
+ * moves stay valid for nested sampling whether or not lnL is periodic in that coordinate.
+ * wrap_bits NULL or all zero: exactly the launches of rvl_slice_phase.  A bit at or above d:
+ * RVL_EINVAL (message in rvl_slice_last_error). */
+int rvl_slice_phase_wrapped(int32_t phase, const rvl_slice_args *args, const uint32_t wrap_bits[4],
+                            void *stream);
 const char *rvl_slice_last_error(void);
 
 #ifdef __cplusplus
