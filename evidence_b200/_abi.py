@@ -66,6 +66,17 @@ class rvl_slice_args(Structure):
                                          "cand", "inside", "cand_ll", "cand_th", "stats")])
 
 
+class rvl_slice_runs(Structure):
+    _fields_ = ([("n_runs", c_int32), ("reserved", c_int32)] +
+                [(n, c_uint64) for n in ("run_of", "walker_of", "seeds", "lmin", "chol", "stats")])
+
+
+class rvl_slice_live(Structure):
+    _fields_ = ([("nlive", c_int32), ("d", c_int32), ("round", ctypes.c_uint32),
+                 ("reserved", ctypes.c_uint32)] +
+                [(n, c_uint64) for n in ("u_live", "th_live", "l_live", "order", "kk", "start", "lstart")])
+
+
 _dp = POINTER(c_double)
 
 # name -> (restype, argtypes); every symbol include/rvlnl.h declares
@@ -127,6 +138,13 @@ SYMBOLS = {
     "rvl_slice_phase": (c_int32, [c_int32, POINTER(rvl_slice_args), c_void_p]),
     "rvl_slice_phase_wrapped": (c_int32, [c_int32, POINTER(rvl_slice_args), POINTER(ctypes.c_uint32),
                                           c_void_p]),
+    "rvl_slice_phase_runs": (c_int32, [c_int32, POINTER(rvl_slice_args), POINTER(rvl_slice_runs),
+                                       POINTER(ctypes.c_uint32), c_void_p]),
+    "rvl_slice_runs_init": (c_int32, [POINTER(rvl_slice_runs), POINTER(rvl_slice_live), c_void_p]),
+    "rvl_slice_runs_whiten": (c_int32, [POINTER(rvl_slice_runs), POINTER(rvl_slice_live),
+                                        POINTER(ctypes.c_uint32), c_void_p]),
+    "rvl_slice_runs_starts": (c_int32, [POINTER(rvl_slice_args), POINTER(rvl_slice_runs),
+                                        POINTER(rvl_slice_live), c_void_p]),
     "rvl_slice_last_error": (c_char_p, []),
     "rvl_plan_describe": (c_int32, [POINTER(c_int32), c_int64, POINTER(c_int64), c_int32]),
 }

@@ -17,6 +17,9 @@ Extra ``ultrasettings`` keys (the "config switch"):
     gets as ``wrapped_params`` -- as circular coordinates; 'ellipsoid' rejects it),
     'postprocess' (False), 'plot' (False)
 
+``run_ensemble`` runs several seeded runs of the built-in device sampler through shared launches and
+writes each as ``run()`` would (one run directory, pickle and ``weighted_post.txt`` per run).
+
 UltraNest is a third-party package that is not part of the reference repository (SURVEY.md 8c).
 When it is importable it is used; otherwise -- or with ``'sampler': 'builtin'`` -- the seeded
 vectorised nested sampler of ``evidence_b200.sampler`` produces ln Z from the same callbacks.
@@ -167,6 +170,15 @@ def run(model, rundict, priordict, ultrasettings=None):
         ti = comm.reduce(ti, op=MPI.MIN, root=0)
         tf = comm.reduce(tf, op=MPI.MAX, root=0)
 
+    return _output(model, rundict, settings, isodate, parnames, name, impl, logz, logzerr, ncall, samples,
+                   ti, tf, t_wall)
+
+
+def _output(model, rundict, settings, isodate, parnames, name, impl, logz, logzerr, ncall, samples,
+            ti, tf, t_wall, evals=None):
+    """The ``Output`` of a run (rank 0; None elsewhere), pickled as ``<file_root>.pkl``: process time
+    tf - ti, wall time t_wall; ``evals``: the lnL evaluations those times cover (default: ncall)."""
+    ndim = len(parnames)
     output = None
     if rank == 0:
         import pandas as pd
@@ -194,7 +206,7 @@ def run(model, rundict, priordict, ultrasettings=None):
         output.samples = pd.DataFrame(np.asarray(samples), columns=parnames)
         if hasattr(model, "counters"):  # observability added by the device path
             output.device_counters = model.counters()
-            output.evals_per_second = output.nlike / max(t_wall, 1e-9)
+            output.evals_per_second = (output.nlike if evals is None else evals) / max(t_wall, 1e-9)
         if "prior_names" in rundict:
             output.priors = rundict["prior_names"]
         if "star_params" in rundict:
@@ -205,6 +217,65 @@ def run(model, rundict, priordict, ultrasettings=None):
             from evidence.post_processing import postprocess  # the reference's own (unchanged)
             postprocess(str(Path(output.base_dir).parent.absolute()))
     return output
+
+
+def run_ensemble(model, rundict, priordict, ultrasettings=None, nruns=4, seeds=None):
+    """
+    ``nruns`` independent runs of the built-in device sampler on ``model`` (the device model, as for
+    ``'builtin_method': 'slice-device'``), advanced together through shared launches
+    (``sampler_dev.nested_sample_ensemble``).  Returns a list of ``Output``: output i is what ``run()``
+    writes for ``rundict['runid'] = f"{runid}_{i}"`` and seed ``seeds[i]`` -- its own pickle, file
+    root and ``run1/chains/weighted_post.txt`` -- so that the reference's post-processing and
+    ``fip_criterion`` (median ln Z over run directories, evidence/fip_criterion.py:245-266) scan
+    them as separately launched runs.  ``seeds`` (default: seed, seed + 1, .. from the settings'
+    'seed', 0 when None) sets nruns.  Every output's runtime, walltime, ``device_counters`` and
+    ``evals_per_second`` (all runs' evaluations over the wall time) are those of the whole ensemble,
+    which is what the GPU did; ``nlike`` is the run's own count.  Settings as for ``run()``;
+    'builtin_wrap' is honoured, and 'postprocess' runs the reference's post-processing on each run's
+    own directory (``<save_dir>/<file_root>``), as ``run()`` does.
+    """
+    from .sampler_dev import nested_sample_ensemble
+    if not hasattr(model, "transform_loglike_device"):
+        raise ValueError("run_ensemble needs the device model (transform_loglike_device)")
+    parnames = model.parnames
+    ndim = len(parnames)
+    isodate = datetime.datetime.today().isoformat()
+    if size > 1:
+        isodate = comm.bcast(isodate, root=0)
+    base = set_ultrasettings(dict(rundict), ultrasettings, ndim, 0, isodate, parnames)
+    if seeds is None:
+        seed0 = 0 if base["seed"] is None else int(base["seed"])
+        seeds = [seed0 + i for i in range(int(nruns))]
+    seeds = [int(s) for s in seeds]
+    wrapped = np.array([("omega" in p) or ("ml0" in p) for p in parnames], dtype=bool)
+    builtin_wrapped = wrapped if base["builtin_wrap"] else None
+    model.set_priors(priordict)
+    ti = time.process_time()
+    t_wall = time.perf_counter()
+    results = nested_sample_ensemble(model.transform_loglike_device, ndim, seeds, nlive=base["nlive"],
+                                     dlogz=base["dlogz"], frac_remain=base["frac_remain"],
+                                     nsteps=base["nsteps"], wrapped=builtin_wrapped,
+                                     device=_torch_device(model), num_bootstraps=base["num_bootstraps"])
+    tf = time.process_time()
+    t_wall = time.perf_counter() - t_wall
+    if size > 1:
+        ti = comm.reduce(ti, op=MPI.MIN, root=0)
+        tf = comm.reduce(tf, op=MPI.MAX, root=0)
+    runid = rundict["runid"].replace(" ", "")
+    outputs = []
+    for i, (seed, res) in enumerate(zip(seeds, results)):
+        rd = dict(rundict, runid=f"{runid}_{i}")
+        settings = set_ultrasettings(rd, ultrasettings, ndim, 0, isodate, parnames)
+        os.makedirs(settings["log_dir"], exist_ok=True)
+        write_weighted_post(settings["log_dir"], parnames, res)
+        impl = (f"evidence_b200.sampler_dev ensemble (slice-device): run {i} of {len(seeds)}, seed {seed}; "
+                "ultranest not used")
+        if builtin_wrapped is not None:
+            impl += "; wrapped: " + (", ".join(p for p, w in zip(parnames, wrapped) if w) or "none")
+        outputs.append(_output(model, rd, settings, isodate, parnames, "UltraNest", impl, res.logz,
+                               res.logzerr, res.ncall, res.samples, ti, tf, t_wall,
+                               evals=sum(r.ncall for r in results)))
+    return outputs
 
 
 def write_weighted_post(log_dir, parnames, res):

@@ -401,6 +401,61 @@ int rvl_slice_phase(int32_t phase, const rvl_slice_args *args, void *stream);
  * RVL_EINVAL (message in rvl_slice_last_error). */
 int rvl_slice_phase_wrapped(int32_t phase, const rvl_slice_args *args, const uint32_t wrap_bits[4],
                             void *stream);
+
+/* An ensemble: R independent runs of one model whose walkers share every launch
+ * (evidence_b200/sampler_dev.py: nested_sample_ensemble).  Walker w of a launch is walker
+ * walker_of[w] of run run_of[w]; the walkers of a run may sit anywhere in the launch.  It uses that
+ * run's constraint lmin[r], whitening chol[r] and counters stats[r], and draws from seeds[r] with
+ * walker_of[w] as the walker word of its counters: exactly what walker j of an rvl_slice_phase call
+ * with k = k_r and seed = seeds[r] draws.  run_of values must lie in [0, n_runs). */
+typedef struct {
+    int32_t n_runs, reserved;
+    uint64_t run_of;    /* const int32_t*  [k]        run of each walker of the launch             */
+    uint64_t walker_of; /* const int32_t*  [k]        its index inside that run                    */
+    uint64_t seeds;     /* const uint64_t* [R]                                                     */
+    uint64_t lmin;      /* const double*   [R]        each run's constraint                        */
+    uint64_t chol;      /* double*         [R][d][d]  each run's whitening (written by _whiten)    */
+    uint64_t stats;     /* uint64_t*       [R][2]     each run's counters, as rvl_slice_args.stats */
+} rvl_slice_runs;
+/* rvl_slice_phase / rvl_slice_phase_wrapped (wrap_bits may be NULL) for the walkers of several runs.
+ * args->k is the total number of walkers; args->seed, lmin, chol and stats are ignored (the runs'
+ * own are used).  Errors as rvl_slice_phase, and RVL_EINVAL for a NULL runs, n_runs < 1 or a
+ * missing address in it. */
+int rvl_slice_phase_runs(int32_t phase, const rvl_slice_args *args, const rvl_slice_runs *runs,
+                         const uint32_t wrap_bits[4], void *stream);
+/* The live points of the R runs of an ensemble, for its set-up calls. */
+typedef struct {
+    int32_t nlive, d;
+    uint32_t round, reserved; /* round: the start draws' counter word (one value per round)    */
+    uint64_t u_live;  /* double*        [R][nlive][d] unit-cube live points                      */
+    uint64_t th_live; /* const double*  [R][nlive][d] their parameters                           */
+    uint64_t l_live;  /* const double*  [R][nlive]    their lnL                                  */
+    uint64_t order;   /* const int64_t* [R][nlive]    each run's points by ascending lnL (a stable sort) */
+    uint64_t kk;      /* const int64_t* [R]           points retired this round, 1 <= kk[r] <= nlive - 2:
+                                                      the survivors of run r are order[r][kk[r]:];
+                                                      0: run r takes no part in the round */
+    uint64_t start;   /* int64_t*       [k]           out: the slot of each walker's start point  */
+    uint64_t lstart;  /* double*        [k]           out: its lnL                                */
+} rvl_slice_live;
+/* The set-up of an ensemble round, each run's values from its own points and seed alone (whatever R):
+ *   _init    u_live[r][p][c] = the uniform of Philox counter (0, 0x494E0000 + c / 2, p, 0) under
+ *            seeds[r] (words x, y for even c; z, w for odd c; the u01 of the slice draws).
+ *            Reads n_runs, seeds, nlive, d, u_live.
+ *   _whiten  one block per run: chol[r] = lower Cholesky factor of 1e-18 I + the covariance of the
+ *            survivors of run r (sums over them in order; divided by n - 1), circular coordinates of
+ *            wrap_bits (may be NULL) first taken modulo 1 about their circular mean, as
+ *            sampler_dev._whitening does; where a pivot is not > 0, diag(sqrt(max(cov_jj, 1e-30))).
+ *            The upper triangle is 0.  A run with kk[r] = 0 is skipped (chol[r] is left as it is).
+ *   _starts  for each walker w of args (k = args->k, run r = run_of[w], j = walker_of[w]): a start
+ *            point, survivor number floor(x n / 2^32) of run r, x the first word of Philox counter
+ *            (round, 0x53540000, j, 0) under seeds[r], n = nlive - kk[r]; copied into args->u and
+ *            args->theta; args->lcur = NaN; start / lstart = its slot and lnL.  args->d == live->d.
+ * Errors: RVL_EINVAL with a message in rvl_slice_last_error for bad sizes or a missing address. */
+int rvl_slice_runs_init(const rvl_slice_runs *runs, const rvl_slice_live *live, void *stream);
+int rvl_slice_runs_whiten(const rvl_slice_runs *runs, const rvl_slice_live *live,
+                          const uint32_t wrap_bits[4], void *stream);
+int rvl_slice_runs_starts(const rvl_slice_args *args, const rvl_slice_runs *runs,
+                          const rvl_slice_live *live, void *stream);
 const char *rvl_slice_last_error(void);
 
 #ifdef __cplusplus
