@@ -145,6 +145,11 @@ SYMBOLS = {
                                         POINTER(ctypes.c_uint32), c_void_p]),
     "rvl_slice_runs_starts": (c_int32, [POINTER(rvl_slice_args), POINTER(rvl_slice_runs),
                                         POINTER(rvl_slice_live), c_void_p]),
+    "rvl_slice_runs_radius": (c_int32, [POINTER(rvl_slice_runs), POINTER(rvl_slice_live),
+                                        POINTER(ctypes.c_uint32), c_void_p, c_void_p]),
+    "rvl_slice_runs_travel": (c_int32, [POINTER(rvl_slice_args), POINTER(rvl_slice_runs),
+                                        POINTER(rvl_slice_live), POINTER(ctypes.c_uint32), c_void_p,
+                                        c_void_p, c_void_p]),
     "rvl_slice_last_error": (c_char_p, []),
     "rvl_plan_describe": (c_int32, [POINTER(c_int32), c_int64, POINTER(c_int64), c_int32]),
 }

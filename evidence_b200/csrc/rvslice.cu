@@ -25,6 +25,9 @@
 // instantiations) shares every launch: walker w belongs to run run_of[w], draws as walker
 // walker_of[w] of that run's seed and reads that run's constraint and whitening, so a run draws
 // what it would draw alone.  rvl_slice_runs_init / _whiten / _starts set up such runs on the device.
+// rvl_slice_runs_radius / _travel measure, per run and round, the largest nearest-neighbour gap of
+// the survivors and how many walkers moved farther than it, in the whitened metric of the moves:
+// the inputs of an adaptive number of moves per run (sampler_dev, adaptive_nsteps='move-distance').
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
@@ -457,6 +460,133 @@ __global__ void __launch_bounds__(128) runs_starts_kernel(const LiveArgs a, int 
     }
 }
 
+// ---- adaptive number of moves: the spacing of each run's survivors and how far its walkers went ------
+// The distance of two unit-cube points a, b under run r's whitening factor L = chol[r]:
+//   D(a, b) = |y|^2,  y = L^-1 delta,  delta = a - b, and delta_c - rint(delta_c) (half to even) in a
+//   circular coordinate.
+// Every value is formed in a fixed order with one rounding per operation (the library is built with
+// -fmad=false and IEEE division), so a host restatement reproduces it bit for bit and a run's values
+// depend on its own points alone, whatever the number of runs:
+//   Linv = L^-1, lower triangular, by forward substitution column by column (thread c forms column c):
+//          Linv_cc = 1 / L_cc;  for i = c + 1 .. d - 1:  s = 0, s = s + L_il Linv_lc for l = c .. i - 1,
+//          Linv_ic = -(s / L_ii)
+//   y_i  = 0, y_i = y_i + Linv_il delta_l for l = 0 .. i
+//   D    = 0, D = D + y_i y_i for i = 0 .. d - 1
+// Linv sits in shared memory, packed by rows (row i at i (i + 1) / 2), and each thread keeps its
+// delta in a shared column (delta_l at l * blockDim.x + threadIdx.x): d <= 128 doubles do not fit in
+// registers.  Minima, maxima and the integer counts are exact, so their order is free.
+constexpr int kAdaptThreads = 128;
+
+struct Wrap4 {
+    uint32_t w[4];  // bit c & 31 of w[c >> 5]: coordinate c is circular
+};
+
+size_t adapt_smem(int d)
+{
+    return ((size_t)d * (d + 1) / 2 + (size_t)kAdaptThreads * d) * sizeof(double);
+}
+
+__device__ __forceinline__ bool circular(const Wrap4 &wr, int c)
+{
+    const uint32_t word = c < 32 ? wr.w[0] : c < 64 ? wr.w[1] : c < 96 ? wr.w[2] : wr.w[3];
+    return ((word >> (c & 31)) & 1u) != 0u;
+}
+
+// Linv of the lower factor L [d][d] (row major) into shared memory; ends with a barrier
+__device__ void form_linv(const double *L, int d, double *Linv)
+{
+    for (int c = threadIdx.x; c < d; c += blockDim.x) {
+        Linv[c * (c + 1) / 2 + c] = 1.0 / L[(size_t)c * d + c];
+        for (int i = c + 1; i < d; ++i) {
+            double s = 0.0;
+            for (int l = c; l < i; ++l) s = s + L[(size_t)i * d + l] * Linv[l * (l + 1) / 2 + c];
+            Linv[i * (i + 1) / 2 + c] = -(s / L[(size_t)i * d + i]);
+        }
+    }
+    __syncthreads();
+}
+
+// D(a, b); dl: this thread's delta column (stride blockDim.x)
+__device__ __forceinline__ double whitened_dist2(const double *a, const double *b, int d, const double *Linv,
+                                                 double *dl, const Wrap4 &wr)
+{
+    const int T = blockDim.x;
+    for (int c = 0; c < d; ++c) {
+        double x = a[c] - b[c];
+        if (circular(wr, c)) x = x - rint(x);
+        dl[c * T] = x;
+    }
+    double D = 0.0;
+    for (int i = 0; i < d; ++i) {
+        const double *row = Linv + i * (i + 1) / 2;
+        double y = 0.0;
+        for (int l = 0; l <= i; ++l) y = y + row[l] * dl[l * T];
+        D = D + y * y;
+    }
+    return D;
+}
+
+// One block per run r with kk[r] > 0 (others are skipped: rad2[r] is left as it is): rad2[r] = the
+// largest nearest-neighbour distance among the survivors u_live[r][order[r][kk[r] + i]], i < n =
+// nlive - kk[r]: max over i of min over j != i of D(u_i, u_j).  Thread t takes i = t, t + T, ..;
+// n < 2: 0.
+__global__ void __launch_bounds__(kAdaptThreads) runs_radius_kernel(const LiveArgs a, const double *chol_all,
+                                                                    const Wrap4 wr, double *rad2)
+{
+    const int r = blockIdx.x, d = a.d;
+    const int64_t kk = a.kk[r];
+    if (kk <= 0) return;
+    extern __shared__ double smem[];
+    __shared__ double wmax[kAdaptThreads / 32];
+    double *Linv = smem, *dl = smem + d * (d + 1) / 2 + threadIdx.x;
+    form_linv(chol_all + (size_t)r * d * d, d, Linv);
+    const int n = a.nlive - (int)kk;
+    const int64_t *rows = a.order + (size_t)r * a.nlive + kk;
+    const double *u = a.u_live + (size_t)r * a.nlive * d;
+    double mx = 0.0;
+    for (int i = threadIdx.x; i < n && n > 1; i += blockDim.x) {
+        const double *ui = u + (size_t)rows[i] * d;
+        double mn = INFINITY;
+        for (int j = 0; j < n; ++j)
+            if (j != i) mn = fmin(mn, whitened_dist2(ui, u + (size_t)rows[j] * d, d, Linv, dl, wr));
+        mx = fmax(mx, mn);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(kFull, mx, o));
+    if ((threadIdx.x & 31) == 0) wmax[threadIdx.x >> 5] = mx;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double m = wmax[0];
+        for (int i = 1; i < (int)(blockDim.x >> 5); ++i) m = fmax(m, wmax[i]);
+        rad2[r] = m;
+    }
+}
+
+// One block per run r with kk[r] > 0 (others are skipped: far[r] is left as it is), one thread per
+// walker w of the launch with run_of[w] == r: far[r] = the number of those with D(u_end[w], u_start[w])
+// > rad2[r], u_end[w] = u[w], u_start[w] = u_live[r][start[w]] (a walker that did not move: D = 0).
+__global__ void __launch_bounds__(kAdaptThreads) runs_travel_kernel(const LiveArgs a, int k, const int32_t *run_of,
+                                                                    const int64_t *start, const double *u,
+                                                                    const double *chol_all, const Wrap4 wr,
+                                                                    const double *rad2, int32_t *far)
+{
+    const int r = blockIdx.x, d = a.d;
+    if (a.kk[r] <= 0) return;
+    extern __shared__ double smem[];
+    __shared__ int count;
+    double *Linv = smem, *dl = smem + d * (d + 1) / 2 + threadIdx.x;
+    if (threadIdx.x == 0) count = 0;
+    form_linv(chol_all + (size_t)r * d * d, d, Linv);
+    const double lim = rad2[r];
+    for (int w = threadIdx.x; w < k; w += blockDim.x) {
+        if (run_of[w] != r) continue;
+        const double *b = a.u_live + ((size_t)r * a.nlive + start[w]) * d;
+        if (whitened_dist2(u + (size_t)w * d, b, d, Linv, dl, wr) > lim) atomicAdd(&count, 1);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) far[r] = count;
+}
+
 int sfail(const std::string &m)
 {
     g_slice_error = m;
@@ -572,6 +702,37 @@ int live_args(const rvl_slice_runs *runs, const rvl_slice_live *l, LiveArgs &a)
     return RVL_OK;
 }
 
+// the common checks of rvl_slice_runs_radius / _travel (seeds are not needed)
+int adapt_args(const rvl_slice_runs *runs, const rvl_slice_live *l, const uint32_t *wrap_bits, const void *rad2,
+               LiveArgs &a, Wrap4 &wr)
+{
+    if (!runs) return sfail("runs is NULL");
+    if (!l) return sfail("live is NULL");
+    if (runs->n_runs < 1 || l->nlive < 3 || l->d <= 0 || l->d > kMaxDim)
+        return sfail("bad sizes (n_runs >= 1, nlive >= 3, 0 < d <= 128)");
+    if (!l->u_live || !l->kk || !runs->chol || !rad2)
+        return sfail("live->u_live, live->kk, runs->chol and rad2 must be set");
+    bool any = false;
+    if (const int rc = read_wrap(wrap_bits, l->d, wr.w, any)) return rc;
+    a.n_runs = runs->n_runs; a.nlive = l->nlive; a.d = l->d; a.round = l->round;
+    a.u_live = (double *)l->u_live; a.order = (const int64_t *)l->order; a.kk = (const int64_t *)l->kk;
+    return RVL_OK;
+}
+
+// lets `kernel` take adapt_smem(d) bytes of dynamic shared memory (up to 197 KB at d = 128)
+template <class K>
+int allow_smem(K kernel, int d)
+{
+    const size_t smem = adapt_smem(d);
+    if (smem <= 48 * 1024) return RVL_OK;
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) {
+        g_slice_error = cudaGetErrorString(e);
+        return RVL_ECUDA;
+    }
+    return RVL_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -640,6 +801,36 @@ int rvl_slice_runs_starts(const rvl_slice_args *s, const rvl_slice_runs *runs, c
     runs_starts_kernel<<<(unsigned)((s->k + wpb - 1) / wpb), wpb * 32, 0, (cudaStream_t)stream>>>(
         a, s->k, (const int32_t *)runs->run_of, (const int32_t *)runs->walker_of, (double *)s->u,
         (double *)s->theta, (double *)s->lcur, (int64_t *)live->start, (double *)live->lstart);
+    return launched();
+}
+
+int rvl_slice_runs_radius(const rvl_slice_runs *runs, const rvl_slice_live *live, const uint32_t wrap_bits[4],
+                          double *rad2, void *stream)
+{
+    LiveArgs a{};
+    Wrap4 wr{};
+    if (const int rc = adapt_args(runs, live, wrap_bits, rad2, a, wr)) return rc;
+    if (!live->order) return sfail("live->order must be set");
+    if (const int rc = allow_smem(runs_radius_kernel, a.d)) return rc;
+    runs_radius_kernel<<<a.n_runs, kAdaptThreads, adapt_smem(a.d), (cudaStream_t)stream>>>(
+        a, (const double *)runs->chol, wr, rad2);
+    return launched();
+}
+
+int rvl_slice_runs_travel(const rvl_slice_args *s, const rvl_slice_runs *runs, const rvl_slice_live *live,
+                          const uint32_t wrap_bits[4], const double *rad2, int32_t *far, void *stream)
+{
+    LiveArgs a{};
+    Wrap4 wr{};
+    if (const int rc = adapt_args(runs, live, wrap_bits, rad2, a, wr)) return rc;
+    if (!s) return sfail("args is NULL");
+    if (s->k <= 0 || s->d != a.d) return sfail("bad sizes (args->k > 0, args->d == live->d)");
+    if (!s->u || !runs->run_of || !live->start || !far)
+        return sfail("travel: args->u, runs->run_of, live->start and far must be set");
+    if (const int rc = allow_smem(runs_travel_kernel, a.d)) return rc;
+    runs_travel_kernel<<<a.n_runs, kAdaptThreads, adapt_smem(a.d), (cudaStream_t)stream>>>(
+        a, s->k, (const int32_t *)runs->run_of, (const int64_t *)live->start, (const double *)s->u,
+        (const double *)runs->chol, wr, rad2, far);
     return launched();
 }
 

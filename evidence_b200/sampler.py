@@ -417,7 +417,8 @@ def _slice_moves(rng, loglike, transform, u, lmin, chol, nsteps, max_expand=16, 
 
 def nested_sample(loglike, transform, ndim, nlive=400, ndraw=4096, dlogz=0.5, frac_remain=0.01,
                   seed=0, nsteps=None, batch_fraction=0.2, method="slice", max_calls=500_000_000,
-                  verbose=False, fused=None, speculate=None, num_bootstraps=30, wrapped=None, **kw):
+                  verbose=False, fused=None, speculate=None, num_bootstraps=30, wrapped=None,
+                  adaptive_nsteps=None, max_nsteps=None, **kw):
     """
     Seeded vectorised nested sampling; see the module docstring.  ``loglike(theta[n, ndim])`` and
     ``transform(u[n, ndim])`` follow UltraNest's ``vectorized=True`` convention.  Returns a
@@ -426,8 +427,13 @@ def nested_sample(loglike, transform, ndim, nlive=400, ndraw=4096, dlogz=0.5, fr
     return what ``transform`` followed by ``loglike`` returns, and then the run is identical.
     ``wrapped`` (bool per dimension, UltraNest's ``wrapped_params``): circular coordinates of the
     slice method (module docstring); None or no True leaves the run exactly as without it.  The
-    result's ``wrapped`` holds the mask.
+    result's ``wrapped`` holds the mask.  ``adaptive_nsteps`` / ``max_nsteps`` (an adaptive number
+    of moves per round) exist on the device samplers only (``sampler_dev``): anything but None is a
+    ValueError here.
     """
+    if adaptive_nsteps is not None or max_nsteps is not None:
+        raise ValueError("adaptive_nsteps / max_nsteps: only the device samplers adapt the number of moves "
+                         "(sampler_dev.nested_sample_device with native kernels, nested_sample_ensemble)")
     wmask = wrap_mask(wrapped, ndim)
     if method == "ellipsoid":
         if wmask.any():

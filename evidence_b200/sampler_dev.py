@@ -13,6 +13,11 @@ sequences the launches and reads back two scalars per round (loop exits).
 runs share every bookkeeping and likelihood launch (``rvl_slice_phase_runs``), each run with its
 own random streams.
 
+Both can adapt each run's number of moves per round (``adaptive_nsteps='move-distance'``, opt-in):
+more moves while most walkers end within the live set's largest nearest-neighbour gap of where they
+started, fewer when most leave it, measured in the moves' whitened metric by
+``rvl_slice_runs_radius`` / ``_travel`` (DESIGN.md section 9.1).
+
 Same algorithm (SURVEY.md 8f row 1; the scheme of PolyChord / UltraNest's step samplers that the
 reference configures at evidence/ultranest/__init__.py:175): per round the k worst live points are
 retired with the shrinkage 1/n for n = nlive, nlive-1, ..; k walkers started from surviving live
@@ -147,6 +152,93 @@ def _slice_moves(torch, gen, fused, u, theta, lmin, chol, nsteps, m, max_expand,
     return u, theta, lcur, ncall
 
 
+def _adaptive_settings(adaptive_nsteps, max_nsteps, nsteps):
+    """(adaptive, cap) for the samplers' ``adaptive_nsteps`` / ``max_nsteps``: None -> (False, nsteps);
+    'move-distance' -> (True, max_nsteps, default 4 nsteps).  Anything else is a ValueError."""
+    if adaptive_nsteps is None:
+        if max_nsteps is not None:
+            raise ValueError("max_nsteps applies with adaptive_nsteps='move-distance' only")
+        return False, nsteps
+    if adaptive_nsteps != "move-distance":
+        raise ValueError(f"adaptive_nsteps: {adaptive_nsteps!r}; None or 'move-distance'")
+    cap = 4 * nsteps if max_nsteps is None else int(max_nsteps)
+    if cap < nsteps:
+        raise ValueError(f"max_nsteps = {cap} is below nsteps = {nsteps}")
+    return True, cap
+
+
+def _adapt_nsteps(n, far, kk, floor, cap):
+    """The next round's moves per walker of each run (int64 arrays over runs): a run whose walkers
+    mostly stayed within the live set's spacing (2 far < kk) makes half as many again (at least one
+    more, at most ``cap``); one whose walkers mostly left it (4 far > 3 kk) a third fewer (at least
+    ``floor``); otherwise the same.  Integer operations only."""
+    n, far, kk = (np.asarray(x, dtype=np.int64) for x in (n, far, kk))
+    up = np.minimum(cap, n + np.maximum(1, n // 2))
+    down = np.maximum(floor, n - n // 3)
+    return np.where(2 * far < kk, up, np.where(4 * far > 3 * kk, down, n))
+
+
+def _move_base(round_no, max_nsteps):
+    """The move number (the Philox counter word) of move 0 of a round with adaptive moves: move j of
+    round i is i * max_nsteps + j whatever a run's own count, so a run's streams do not depend on the
+    other runs.  OverflowError where the round's last move would not fit 32 bits."""
+    if (round_no + 1) * max_nsteps - 1 > 0xFFFFFFFF:
+        raise OverflowError(f"round {round_no} x max_nsteps {max_nsteps}: the move number exceeds 32 bits")
+    return round_no * max_nsteps
+
+
+def _adaptive_layout(counts, n_r):
+    """(run_of, walker_of, ks) of a round with per-run move counts n_r: runs sorted by n_r, descending
+    (ties in run order), the walkers of each run as in ``_walker_layout``; ks[j], j < max n_r of the
+    runs with walkers: the walkers whose run makes more than j moves, which are the first ks[j]."""
+    counts, n_r = np.asarray(counts, dtype=np.int64), np.asarray(n_r, dtype=np.int64)
+    runs = np.argsort(-n_r, kind="stable")
+    pos, walker_of = _walker_layout(counts[runs])
+    run_of = runs[pos].astype(np.int32)
+    busy = counts > 0
+    top = int(n_r[busy].max()) if busy.any() else 0
+    ks = [int(counts[n_r > j].sum()) for j in range(top)]
+    return run_of, walker_of, ks
+
+
+class _Travel:
+    """``rvl_slice_runs_radius`` / ``_travel`` for the single-run sampler: one run (n_runs = 1), the
+    far walkers' count in ``far[0]``."""
+
+    def __init__(self, torch, nlive, d, dev, wrap):
+        import ctypes
+        from . import _abi
+        self.lib = _abi.load()
+        self.rad2 = torch.zeros(1, dtype=torch.float64, device=dev)
+        self.far = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.kk = torch.zeros(1, dtype=torch.int64, device=dev)
+        self.run_of = torch.zeros(nlive, dtype=torch.int32, device=dev)  # walkers of a round: <= nlive - 2
+        self.runs = _abi.rvl_slice_runs(n_runs=1, run_of=self.run_of.data_ptr())
+        self.live = _abi.rvl_slice_live(nlive=nlive, d=d, kk=self.kk.data_ptr())
+        self._runs, self._live = ctypes.byref(self.runs), ctypes.byref(self.live)
+        self.wrap_bits = _wrap_bits(wrap)
+
+    def measure(self, torch, u_live, order, kk, chol, starts, args):
+        """rad2 of the survivors order[kk:] of u_live, then far = the walkers of ``args`` (its u,
+        started from u_live[starts]) that moved farther, under the whitening ``chol``."""
+        import ctypes
+        chol = chol.contiguous()
+        self.kk.fill_(kk)
+        self.runs.chol = chol.data_ptr()
+        self.live.u_live, self.live.order, self.live.start = u_live.data_ptr(), order.data_ptr(), starts.data_ptr()
+        stream = torch.cuda.current_stream().cuda_stream
+        _check_slice(self.lib, self.lib.rvl_slice_runs_radius(self._runs, self._live, self.wrap_bits,
+                                                              self.rad2.data_ptr(), stream), "rvl_slice_runs_radius")
+        _check_slice(self.lib, self.lib.rvl_slice_runs_travel(ctypes.byref(args), self._runs, self._live,
+                                                              self.wrap_bits, self.rad2.data_ptr(),
+                                                              self.far.data_ptr(), stream), "rvl_slice_runs_travel")
+
+
+def _check_slice(lib, rc, what):
+    if rc != 0:
+        raise RuntimeError(f"{what}: " + lib.rvl_slice_last_error().decode())
+
+
 def _wrap_bits(wrap):
     """The mask of rvl_slice_phase_wrapped (uint32[4]) for a bool per dimension; None without a True."""
     import ctypes
@@ -248,7 +340,8 @@ class _NativeSlice:
 def nested_sample_device(fused, ndim, nlive=400, dlogz=0.5, frac_remain=0.01, seed=0, nsteps=None,
                          batch_fraction=0.2, speculate=None, device="cuda", max_expand=16,
                          max_shrink=64, max_calls=2_000_000_000, verbose=False, num_bootstraps=30,
-                         native=None, native_m=8, native_rounds=3, native_out=8, wrapped=None):
+                         native=None, native_m=8, native_rounds=3, native_out=8, wrapped=None,
+                         adaptive_nsteps=None, max_nsteps=None):
     """
     Nested sampling with every array on ``device``.  ``fused(U[n, ndim]) -> (theta[n, ndim],
     lnL[n])`` maps unit-cube points to parameters and log-likelihoods on that device
@@ -263,6 +356,14 @@ def nested_sample_device(fused, ndim, nlive=400, dlogz=0.5, frac_remain=0.01, se
 
     ``wrapped`` (bool per dimension, UltraNest's ``wrapped_params``): circular coordinates, as in
     ``sampler.nested_sample``; None or no True leaves the run exactly as without it.
+
+    ``adaptive_nsteps='move-distance'`` (native kernels only): the number of moves per walker starts
+    at ``nsteps`` and is adapted after every round by the rule of ``_adapt_nsteps`` between
+    ``nsteps`` and ``max_nsteps`` (default 4 nsteps), from how many walkers ended farther from their
+    start than the largest nearest-neighbour gap of the survivors, both in the moves' whitened metric
+    (``rvl_slice_runs_radius`` / ``_travel``).  Move j of round i then draws with move number
+    i * max_nsteps + j.  The result's ``nsteps_history`` lists the count of every round.  None: the
+    fixed ``nsteps`` of before, exactly.
     """
     import torch
     dev = torch.device(device)
@@ -271,6 +372,9 @@ def nested_sample_device(fused, ndim, nlive=400, dlogz=0.5, frac_remain=0.01, se
     if native is None:
         native = dev.type == "cuda"
     nsteps = nsteps or max(4, 3 * ndim)  # the reference's default (evidence/ultranest/__init__.py:335)
+    adaptive, cap = _adaptive_settings(adaptive_nsteps, max_nsteps, nsteps)
+    if adaptive and not native:
+        raise ValueError("adaptive_nsteps needs the native kernels (native=True, a CUDA device)")
     wmask = wrap_mask(wrapped, ndim)
     wrap = torch.as_tensor(wmask, device=dev) if wmask.any() else None
     k = max(1, min(int(batch_fraction * nlive), nlive - 2))
@@ -294,6 +398,8 @@ def nested_sample_device(fused, ndim, nlive=400, dlogz=0.5, frac_remain=0.01, se
     dead_root, dead_birth = [], []
     niter = 0
     natives, move_no = {}, 0
+    if adaptive:
+        probe, n_cur, history, round_no = _Travel(torch, nlive, ndim, dev, wmask), nsteps, [], 0
     l_sorted, order = torch.sort(l_live, stable=True)
     # points tied with the k-th worst are retired with it (a plateau goes as a whole: retire_groups);
     # the count rides on the one read-back per round
@@ -321,11 +427,16 @@ def nested_sample_device(fused, ndim, nlive=400, dlogz=0.5, frac_remain=0.01, se
             if kk not in natives:
                 natives[kk] = _NativeSlice(torch, kk, ndim, dev, seed, n_out=native_out, m=native_m,
                                            rounds=native_rounds, wrap=wmask)
-            natives[kk].move = move_no
+            natives[kk].move = _move_base(round_no, cap) if adaptive else move_no
             u_new, th_new = u_live[starts].clone(), th_live[starts].clone()
             l_new = torch.full((kk,), float("nan"), dtype=f64, device=dev)
-            nc = natives[kk].moves(fused, u_new, th_new, l_new, lmin.reshape(1).clone(), chol, nsteps)
+            nc = natives[kk].moves(fused, u_new, th_new, l_new, lmin.reshape(1).clone(), chol,
+                                   n_cur if adaptive else nsteps)
             move_no += nsteps
+            if adaptive:
+                history.append(n_cur)
+                probe.measure(torch, u_live, order, kk, chol, starts, natives[kk].args)
+                round_no += 1
         else:
             u_new, th_new, l_new, nc = _slice_moves(torch, gen, fused, u_live[starts].clone(),
                                                     th_live[starts].clone(), lmin, chol, nsteps, m,
@@ -342,7 +453,12 @@ def nested_sample_device(fused, ndim, nlive=400, dlogz=0.5, frac_remain=0.01, se
         log_remain = l_sorted[-1] + logx
         total = torch.logaddexp(logz, log_remain)
         tied = (l_sorted <= l_sorted[k - 1]).sum().to(f64)
-        lr, tt, lz, kk = (float(x) for x in torch.stack([log_remain, total, logz, tied]).cpu())
+        if adaptive:  # the far walkers' count rides on the same read-back
+            back = torch.stack([log_remain, total, logz, tied, probe.far[0].to(f64)]).cpu().numpy()
+            n_cur = int(_adapt_nsteps([n_cur], [int(back[4])], [kk], nsteps, cap)[0])
+            lr, tt, lz, kk = (float(x) for x in back[:4])
+        else:
+            lr, tt, lz, kk = (float(x) for x in torch.stack([log_remain, total, logz, tied]).cpu())
         kk = int(kk)
         if verbose and (niter // k) % 20 == 0:
             print(f"it={niter} lnZ={lz:.3f} ln(remain/Z)={lr - lz:.2f} ncall={ncall}")
@@ -370,15 +486,18 @@ def nested_sample_device(fused, ndim, nlive=400, dlogz=0.5, frac_remain=0.01, se
     bs_std, _ = lineage_bootstrap(torch.cat(dead_birth).cpu().numpy(), logl.cpu().numpy(),
                                   torch.cat(dead_root).cpu().numpy(), nlive,
                                   np.random.default_rng([int(seed), 0xB007]), num_bootstraps)
-    return NestedResult(logz=float(logz), logzerr=float(max(skilling, bs_std)),
-                        logzerr_skilling=skilling, logzerr_bootstrap=bs_std,
-                        ncall=int(ncall), niter=int(niter), information=h_info,
-                        samples=theta[idx].cpu().numpy(), weighted_samples=theta.cpu().numpy(),
-                        weights=weights.cpu().numpy(), logl=logl.cpu().numpy(), nlive=nlive,
-                        seed=seed, method="slice-device" + ("-native" if native else ""),
-                        unresolved_moves=int(sum(int(n.stats[0]) for n in natives.values())),
-                        accepted_moves=int(sum(int(n.stats[1]) for n in natives.values())),
-                        wrapped=wmask)
+    res = NestedResult(logz=float(logz), logzerr=float(max(skilling, bs_std)),
+                       logzerr_skilling=skilling, logzerr_bootstrap=bs_std,
+                       ncall=int(ncall), niter=int(niter), information=h_info,
+                       samples=theta[idx].cpu().numpy(), weighted_samples=theta.cpu().numpy(),
+                       weights=weights.cpu().numpy(), logl=logl.cpu().numpy(), nlive=nlive,
+                       seed=seed, method="slice-device" + ("-native" if native else ""),
+                       unresolved_moves=int(sum(int(n.stats[0]) for n in natives.values())),
+                       accepted_moves=int(sum(int(n.stats[1]) for n in natives.values())),
+                       wrapped=wmask)
+    if adaptive:
+        res["nsteps_history"] = history
+    return res
 
 
 # ------------------------------------------------------------------------------------------------
@@ -493,10 +612,30 @@ class _NativeSliceRuns(_NativeSlice):
         self._check(self.lib.rvl_slice_runs_starts(self._byref, self._runs, self._live, self._stream()),
                     "rvl_slice_runs_starts")
 
+    def moves_prefix(self, fused, lmin, ks):
+        """Adaptive moves of a round laid out by ``_adaptive_layout``: move j launches the first ks[j]
+        walkers only (args.k and the candidate buffers cut to them); the full layout is restored."""
+        k = self.k
+        for kj in ks:
+            self.reserve(kj)
+            self.moves(fused, self.u, self.theta, self.lcur, lmin, self.chol, 1)
+        self.reserve(k)
+
+    def radius(self, rad2):
+        """rad2[r] = the largest nearest-neighbour gap of run r's survivors (runs with kk = 0 kept)."""
+        self._check(self.lib.rvl_slice_runs_radius(self._runs, self._live, self.wrap_bits, rad2.data_ptr(),
+                                                   self._stream()), "rvl_slice_runs_radius")
+
+    def travel(self, rad2, far):
+        """far[r] = the walkers of run r that ended farther than rad2[r] from their start."""
+        self._check(self.lib.rvl_slice_runs_travel(self._byref, self._runs, self._live, self.wrap_bits,
+                                                   rad2.data_ptr(), far.data_ptr(), self._stream()),
+                    "rvl_slice_runs_travel")
+
 
 def nested_sample_ensemble(fused, ndim, seeds, nlive=400, dlogz=0.5, frac_remain=0.01, nsteps=None,
                            wrapped=None, device="cuda", native_m=8, native_rounds=3, native_out=8,
-                           num_bootstraps=30, max_calls=2_000_000_000):
+                           num_bootstraps=30, max_calls=2_000_000_000, adaptive_nsteps=None, max_nsteps=None):
     """
     R = len(seeds) independent runs of ``nested_sample_device`` (native kernels, batch_fraction 0.2)
     on one likelihood, advanced in lockstep: every bookkeeping launch and every likelihood launch
@@ -516,6 +655,12 @@ def nested_sample_ensemble(fused, ndim, seeds, nlive=400, dlogz=0.5, frac_remain
 
     The host reads back one [R, 4] tensor per round (loop exits and tie counts), plus the retired
     values of a run in a plateau round (``retire_groups``), as the single-run sampler does.
+
+    ``adaptive_nsteps='move-distance'``: each run adapts its own number of moves as
+    ``nested_sample_device`` does (same rule, same move numbers, its ``nsteps_history``), from its own
+    points and walkers alone.  A round lays the walkers out with runs sorted by their count,
+    descending (``_adaptive_layout``), so that move j launches only the walkers still moving, a
+    prefix.  The far walkers' counts ride on the round's read-back as a fifth column.
     """
     import torch
     seeds = _ensemble_seeds(seeds)
@@ -525,8 +670,10 @@ def nested_sample_ensemble(fused, ndim, seeds, nlive=400, dlogz=0.5, frac_remain
         raise ValueError("nested_sample_ensemble runs the kernels of csrc/rvslice.cu: device must be CUDA")
     R, f64 = len(seeds), torch.float64
     nsteps = nsteps or max(4, 3 * ndim)
+    adaptive, cap = _adaptive_settings(adaptive_nsteps, max_nsteps, nsteps)
     k = max(1, min(int(0.2 * nlive), nlive - 2))
-    per_walker = nsteps * (2 * native_out + native_rounds * native_m)  # lnL calls per walker and round
+    per_move = 2 * native_out + native_rounds * native_m  # lnL calls per walker and move
+    per_walker = nsteps * per_move  # lnL calls per walker and round
     ns = _NativeSliceRuns(torch, ndim, dev, seeds, nlive, n_out=native_out, m=native_m,
                           rounds=native_rounds, wrap=wmask)
     u_live = ns.init()
@@ -554,6 +701,11 @@ def nested_sample_ensemble(fused, ndim, seeds, nlive=400, dlogz=0.5, frac_remain
     up_f = torch.empty(2 * R, dtype=f64).pin_memory()
     dev_i = torch.empty(up_i.shape, dtype=torch.int32, device=dev)
     dev_f = torch.empty(up_f.shape, dtype=f64, device=dev)
+    if adaptive:
+        n_r = np.full(R, nsteps, dtype=np.int64)
+        history = [[] for _ in range(R)]
+        rad2 = torch.zeros(R, dtype=f64, device=dev)
+        far = torch.zeros(R, dtype=torch.int32, device=dev)
     while active.any():
         act = np.flatnonzero(active)
         kk = np.minimum(kk, nlive - 2)
@@ -567,7 +719,10 @@ def nested_sample_ensemble(fused, ndim, seeds, nlive=400, dlogz=0.5, frac_remain
         niter[act] += kk[act]
         # the round's walkers: kk[r] for every active run, walker j of run r replaces order[r][j]
         counts = np.where(active, kk, 0)
-        run_of, walker_of = _walker_layout(counts)
+        if adaptive:
+            run_of, walker_of, ks = _adaptive_layout(counts, n_r)
+        else:
+            run_of, walker_of = _walker_layout(counts)
         K, G = len(run_of), len(regular)
         n_up = R + 2 * K + G
         up_i[:n_up] = torch.from_numpy(np.concatenate([counts.astype(np.int32), run_of, walker_of,
@@ -596,11 +751,20 @@ def nested_sample_ensemble(fused, ndim, seeds, nlive=400, dlogz=0.5, frac_remain
         ns.reserve(K)
         lmin = l_sorted.gather(1, (kk_dev - 1).clamp(min=0)[:, None]).reshape(R)
         ns.setup_round(th_live, l_live, order, kk_dev, lmin, run_t, walker_t, round_no)
-        ns.move = move_no
-        ns.moves(fused, ns.u, ns.theta, ns.lcur, lmin, ns.chol, nsteps)
+        if adaptive:
+            ns.radius(rad2)
+            ns.move = _move_base(round_no, cap)
+            ns.moves_prefix(fused, lmin, ks)
+            ns.travel(rad2, far)
+            ncall += counts * n_r * per_move
+            for r in act:
+                history[r].append(int(n_r[r]))
+        else:
+            ns.move = move_no
+            ns.moves(fused, ns.u, ns.theta, ns.lcur, lmin, ns.chol, nsteps)
+            ncall += counts * per_walker
         move_no += nsteps
         round_no += 1
-        ncall += counts * per_walker
         stuck = ~torch.isfinite(ns.lcur)  # a walker that never moved is a copy of its start point
         l_new = torch.where(stuck, ns.lstart, ns.lcur)
         run_l = run_t.long()
@@ -615,7 +779,10 @@ def nested_sample_ensemble(fused, ndim, seeds, nlive=400, dlogz=0.5, frac_remain
         log_remain = l_sorted[:, -1] + dev_f[R:]
         total = torch.logaddexp(logz, log_remain)
         tied = (l_sorted <= l_sorted[:, k - 1:k]).sum(1).to(f64)
-        back = torch.stack([log_remain, total, logz, tied], 1).cpu().numpy()  # one read-back per round
+        cols = [log_remain, total, logz, tied] + ([far.to(f64)] if adaptive else [])
+        back = torch.stack(cols, 1).cpu().numpy()  # one read-back per round
+        if adaptive:
+            n_r[act] = _adapt_nsteps(n_r[act], back[act, 4].astype(np.int64), counts[act], nsteps, cap)
         kk = back[:, 3].astype(np.int64)
         for r in act:
             lr, tt, lz = back[r, :3]
@@ -628,10 +795,11 @@ def nested_sample_ensemble(fused, ndim, seeds, nlive=400, dlogz=0.5, frac_remain
                                 root_live[r, o][None], birth_live[r, o][None]))
                 active[r] = False
     return _ensemble_results(records, logz.cpu().numpy(), ns.stats.cpu().numpy(), seeds, ncall, niter,
-                             nlive, ndim, wmask, num_bootstraps)
+                             nlive, ndim, wmask, num_bootstraps, history if adaptive else None)
 
 
-def _ensemble_results(records, logz, stats, seeds, ncall, niter, nlive, ndim, wmask, num_bootstraps):
+def _ensemble_results(records, logz, stats, seeds, ncall, niter, nlive, ndim, wmask, num_bootstraps,
+                      history=None):
     """One NestedResult per run from the retirement records of an ensemble (host numpy; each run's
     arrays in the order its points died, as nested_sample_device keeps them)."""
     import torch
@@ -665,4 +833,6 @@ def _ensemble_results(records, logz, stats, seeds, ncall, niter, nlive, ndim, wm
                                 method="slice-device-native-ensemble",
                                 unresolved_moves=int(stats[r, 0]), accepted_moves=int(stats[r, 1]),
                                 wrapped=wmask))
+        if history is not None:
+            out[-1]["nsteps_history"] = history[r]
     return out

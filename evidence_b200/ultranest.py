@@ -15,6 +15,9 @@ Extra ``ultrasettings`` keys (the "config switch"):
     'sampler' ('auto' | 'ultranest' | 'builtin'), 'builtin_method' ('slice' | 'slice-device' | 'ellipsoid'),
     'builtin_wrap' (False: the built-in slice samplers take the wrapped parameters -- the ones UltraNest
     gets as ``wrapped_params`` -- as circular coordinates; 'ellipsoid' rejects it),
+    'builtin_adaptive_nsteps' (False | 'move-distance': the device sampler adapts each run's number of
+    moves per round, ``sampler_dev.nested_sample_device(adaptive_nsteps=...)``; 'slice-device' and
+    ``run_ensemble`` only, 'slice' and 'ellipsoid' reject it),
     'postprocess' (False), 'plot' (False)
 
 ``run_ensemble`` runs several seeded runs of the built-in device sampler through shared launches and
@@ -139,6 +142,10 @@ def run(model, rundict, priordict, ultrasettings=None):
         fused = getattr(model, "transform_loglike_batch", None) if hasattr(model, "set_priors") else None
         # the circular parameters UltraNest gets, only when asked for
         builtin_wrapped = wrapped if settings["builtin_wrap"] else None
+        adaptive = _adaptive_setting(settings)
+        if adaptive is not None and settings["builtin_method"] != "slice-device":
+            raise ValueError(f"'builtin_adaptive_nsteps': {adaptive!r} needs 'builtin_method': 'slice-device', "
+                             f"not {settings['builtin_method']!r}")
         if settings["builtin_method"] == "slice-device":
             # the whole run on the likelihood's device (evidence_b200.sampler_dev)
             from .sampler_dev import nested_sample_device
@@ -148,7 +155,8 @@ def run(model, rundict, priordict, ultrasettings=None):
                                        nlive=settings["nlive"], dlogz=settings["dlogz"],
                                        frac_remain=settings["frac_remain"], nsteps=settings["nsteps"],
                                        seed=0 if settings["seed"] is None else settings["seed"],
-                                       device=_torch_device(model), wrapped=builtin_wrapped)
+                                       device=_torch_device(model), wrapped=builtin_wrapped,
+                                       adaptive_nsteps=adaptive)
         else:
             res = nested_sample(loglike, prior, ndim, nlive=settings["nlive"], fused=fused,
                                 ndraw=settings["ndraw_min"], dlogz=settings["dlogz"],
@@ -163,6 +171,8 @@ def run(model, rundict, priordict, ultrasettings=None):
         impl = f"evidence_b200.sampler ({settings['builtin_method']}); ultranest not used"
         if builtin_wrapped is not None:
             impl += "; wrapped: " + (", ".join(p for p, w in zip(parnames, wrapped) if w) or "none")
+        if adaptive is not None:
+            impl += _nsteps_note(adaptive, res.nsteps_history)
         write_weighted_post(settings["log_dir"], parnames, res)
     tf = time.process_time()
     t_wall = time.perf_counter() - t_wall
@@ -170,14 +180,16 @@ def run(model, rundict, priordict, ultrasettings=None):
         ti = comm.reduce(ti, op=MPI.MIN, root=0)
         tf = comm.reduce(tf, op=MPI.MAX, root=0)
 
+    history = res.nsteps_history if which != "ultranest" else None
     return _output(model, rundict, settings, isodate, parnames, name, impl, logz, logzerr, ncall, samples,
-                   ti, tf, t_wall)
+                   ti, tf, t_wall, nsteps_history=history)
 
 
 def _output(model, rundict, settings, isodate, parnames, name, impl, logz, logzerr, ncall, samples,
-            ti, tf, t_wall, evals=None):
+            ti, tf, t_wall, evals=None, nsteps_history=None):
     """The ``Output`` of a run (rank 0; None elsewhere), pickled as ``<file_root>.pkl``: process time
-    tf - ti, wall time t_wall; ``evals``: the lnL evaluations those times cover (default: ncall)."""
+    tf - ti, wall time t_wall; ``evals``: the lnL evaluations those times cover (default: ncall);
+    ``nsteps_history``: the moves per round of an adaptive run (set as an attribute when given)."""
     ndim = len(parnames)
     output = None
     if rank == 0:
@@ -204,6 +216,8 @@ def _output(model, rundict, settings, isodate, parnames, name, impl, logz, logze
         output.logZerr = float(logzerr)
         output.nlike = int(ncall)
         output.samples = pd.DataFrame(np.asarray(samples), columns=parnames)
+        if nsteps_history is not None:
+            output.nsteps_history = list(nsteps_history)
         if hasattr(model, "counters"):  # observability added by the device path
             output.device_counters = model.counters()
             output.evals_per_second = (output.nlike if evals is None else evals) / max(t_wall, 1e-9)
@@ -231,8 +245,8 @@ def run_ensemble(model, rundict, priordict, ultrasettings=None, nruns=4, seeds=N
     'seed', 0 when None) sets nruns.  Every output's runtime, walltime, ``device_counters`` and
     ``evals_per_second`` (all runs' evaluations over the wall time) are those of the whole ensemble,
     which is what the GPU did; ``nlike`` is the run's own count.  Settings as for ``run()``;
-    'builtin_wrap' is honoured, and 'postprocess' runs the reference's post-processing on each run's
-    own directory (``<save_dir>/<file_root>``), as ``run()`` does.
+    'builtin_wrap' and 'builtin_adaptive_nsteps' are honoured, and 'postprocess' runs the reference's
+    post-processing on each run's own directory (``<save_dir>/<file_root>``), as ``run()`` does.
     """
     from .sampler_dev import nested_sample_ensemble
     if not hasattr(model, "transform_loglike_device"):
@@ -249,13 +263,15 @@ def run_ensemble(model, rundict, priordict, ultrasettings=None, nruns=4, seeds=N
     seeds = [int(s) for s in seeds]
     wrapped = np.array([("omega" in p) or ("ml0" in p) for p in parnames], dtype=bool)
     builtin_wrapped = wrapped if base["builtin_wrap"] else None
+    adaptive = _adaptive_setting(base)
     model.set_priors(priordict)
     ti = time.process_time()
     t_wall = time.perf_counter()
     results = nested_sample_ensemble(model.transform_loglike_device, ndim, seeds, nlive=base["nlive"],
                                      dlogz=base["dlogz"], frac_remain=base["frac_remain"],
                                      nsteps=base["nsteps"], wrapped=builtin_wrapped,
-                                     device=_torch_device(model), num_bootstraps=base["num_bootstraps"])
+                                     device=_torch_device(model), num_bootstraps=base["num_bootstraps"],
+                                     adaptive_nsteps=adaptive)
     tf = time.process_time()
     t_wall = time.perf_counter() - t_wall
     if size > 1:
@@ -272,10 +288,30 @@ def run_ensemble(model, rundict, priordict, ultrasettings=None, nruns=4, seeds=N
                 "ultranest not used")
         if builtin_wrapped is not None:
             impl += "; wrapped: " + (", ".join(p for p, w in zip(parnames, wrapped) if w) or "none")
+        if adaptive is not None:
+            impl += _nsteps_note(adaptive, res.nsteps_history)
         outputs.append(_output(model, rd, settings, isodate, parnames, "UltraNest", impl, res.logz,
                                res.logzerr, res.ncall, res.samples, ti, tf, t_wall,
-                               evals=sum(r.ncall for r in results)))
+                               evals=sum(r.ncall for r in results), nsteps_history=res.nsteps_history))
     return outputs
+
+
+def _adaptive_setting(settings):
+    """The samplers' ``adaptive_nsteps`` for the setting 'builtin_adaptive_nsteps': None when it is
+    False or None, 'move-distance' as is; anything else is a ValueError."""
+    value = settings["builtin_adaptive_nsteps"]
+    if value is False or value is None:
+        return None
+    if value != "move-distance":
+        raise ValueError(f"'builtin_adaptive_nsteps': {value!r}; False or 'move-distance'")
+    return value
+
+
+def _nsteps_note(adaptive, history):
+    """The implementation string's note on the adapted number of moves per round."""
+    h = np.asarray(history)
+    return (f"; adaptive nsteps ({adaptive}): moves per round min {h.min()}, median {np.median(h):g}, "
+            f"max {h.max()} over {len(h)} rounds")
 
 
 def write_weighted_post(log_dir, parnames, res):
@@ -309,7 +345,7 @@ def set_ultrasettings(rundict, ultrasettings, ndim, nderived, isodate, parnames)
                 # the device-path switch
                 "vectorized": True, "ndraw_min": 4096, "ndraw_max": 65536, "seed": None,
                 "stepsampler": "region-slice", "sampler": "auto", "builtin_method": "slice",
-                "builtin_wrap": False,
+                "builtin_wrap": False, "builtin_adaptive_nsteps": False,
                 "postprocess": False, "plot": False}
     if ultrasettings is not None:
         if type(ultrasettings) is not dict:

@@ -456,6 +456,27 @@ int rvl_slice_runs_whiten(const rvl_slice_runs *runs, const rvl_slice_live *live
                           const uint32_t wrap_bits[4], void *stream);
 int rvl_slice_runs_starts(const rvl_slice_args *args, const rvl_slice_runs *runs,
                           const rvl_slice_live *live, void *stream);
+/* The inputs of an adaptive number of moves per run (sampler_dev: adaptive_nsteps='move-distance'),
+ * each run's values from its own points alone (whatever R) and bit-reproducible.  The distance of
+ * two unit-cube points under run r's whitening L = chol[r] (the factor the moves use) is
+ * D(a, b) = |L^-1 delta|^2, delta = a - b, with delta_c - rint(delta_c) (half to even) in a circular
+ * coordinate of wrap_bits (may be NULL).  L^-1 by forward substitution column by column, y_i and
+ * D = sum y_i^2 as sums in ascending index, one rounding per operation (csrc/rvslice.cu states the
+ * order).  One block per run; a run with kk[r] = 0 is skipped (its output is left as it is).
+ *   _radius  rad2[r] (double*, device, [R]) = max over the survivors i of run r of min over the other
+ *            survivors j of D(u_i, u_j): the largest nearest-neighbour gap of the live set in the
+ *            moves' metric; 0 with fewer than two survivors.  Reads n_runs, chol, nlive, d, u_live,
+ *            order, kk.
+ *   _travel  far[r] (int32_t*, device, [R]) = the number of walkers w of args (k = args->k, r =
+ *            run_of[w]) with D(u_end, u_start) > rad2[r], u_end = args->u[w] and u_start =
+ *            u_live[r][start[w]] (the survivor it started from; a walker that never moved has
+ *            travelled 0).  Counted with integer atomics: exact.  args->d == live->d.
+ * A single run uses them with n_runs = 1 (run_of all 0).  Errors: RVL_EINVAL with a message in
+ * rvl_slice_last_error for bad sizes or a missing address. */
+int rvl_slice_runs_radius(const rvl_slice_runs *runs, const rvl_slice_live *live, const uint32_t wrap_bits[4],
+                          double *rad2, void *stream);
+int rvl_slice_runs_travel(const rvl_slice_args *args, const rvl_slice_runs *runs, const rvl_slice_live *live,
+                          const uint32_t wrap_bits[4], const double *rad2, int32_t *far, void *stream);
 const char *rvl_slice_last_error(void);
 
 #ifdef __cplusplus
