@@ -77,6 +77,13 @@ class rvl_slice_live(Structure):
                 [(n, c_uint64) for n in ("u_live", "th_live", "l_live", "order", "kk", "start", "lstart")])
 
 
+class rvl_region_args(Structure):
+    _fields_ = ([("num_bootstraps", c_int32), ("batch", ctypes.c_uint32), ("max_slots", c_int32),
+                 ("reserved", c_int32)] +
+                [(n, c_uint64) for n in ("rad2", "slot_base", "stage", "flag", "count", "offs", "cand", "cand_th",
+                                         "cand_ll", "sel", "filled", "above")])
+
+
 _dp = POINTER(c_double)
 
 # name -> (restype, argtypes); every symbol include/rvlnl.h declares
@@ -150,6 +157,12 @@ SYMBOLS = {
     "rvl_slice_runs_travel": (c_int32, [POINTER(rvl_slice_args), POINTER(rvl_slice_runs),
                                         POINTER(rvl_slice_live), POINTER(ctypes.c_uint32), c_void_p,
                                         c_void_p, c_void_p]),
+    "rvl_region_runs_radius": (c_int32, [POINTER(rvl_region_args), POINTER(rvl_slice_runs),
+                                         POINTER(rvl_slice_live), POINTER(ctypes.c_uint32), c_void_p]),
+    "rvl_region_runs_draw": (c_int32, [POINTER(rvl_region_args), POINTER(rvl_slice_runs),
+                                       POINTER(rvl_slice_live), POINTER(ctypes.c_uint32), c_void_p]),
+    "rvl_region_runs_pick": (c_int32, [POINTER(rvl_region_args), POINTER(rvl_slice_args),
+                                       POINTER(rvl_slice_runs), POINTER(rvl_slice_live), c_void_p]),
     "rvl_slice_last_error": (c_char_p, []),
     "rvl_plan_describe": (c_int32, [POINTER(c_int32), c_int64, POINTER(c_int64), c_int32]),
 }

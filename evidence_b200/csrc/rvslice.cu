@@ -28,6 +28,8 @@
 // rvl_slice_runs_radius / _travel measure, per run and round, the largest nearest-neighbour gap of
 // the survivors and how many walkers moved farther than it, in the whitened metric of the moves:
 // the inputs of an adaptive number of moves per run (sampler_dev, adaptive_nsteps='move-distance').
+// rvl_region_runs_radius / _draw / _pick fill a round's walkers of each run by MLFriends region sampling
+// instead: independent draws from the union of balls around the survivors (sampler_dev, method='mlfriends').
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
@@ -587,6 +589,236 @@ __global__ void __launch_bounds__(kAdaptThreads) runs_travel_kernel(const LiveAr
     if (threadIdx.x == 0) far[r] = count;
 }
 
+// ---- MLFriends region sampling of an ensemble: independent draws from the constrained prior ------
+// The region of run r is the union of the balls D(x, u_i) <= rho2[r] around its survivors u_i
+// (order[r][kk[r] + i], i < n), D the distance of whitened_dist2 under chol[r].  Counter layout (the
+// c0 word is the round, live->round, as for the starts; every tag below is used by no other kernel):
+//   (round, kTagBoot + b, q, 0)                 bootstrap b: survivor indices 4q .. 4q + 3 of the draw
+//                                               with replacement, floor(word n / 2^32) of words x, y, z, w
+//   (round, kTagRegion + (batch << 8), s, 0)    candidate slot s of a batch: survivor floor(x n / 2^32)
+//                                               and v = u01(z, w)
+//   (round, kTagRegion + (batch << 8) + 1 + (c >> 1), s, 0)
+//                                               its Gaussian coordinate c: Box-Muller of u01(x, y),
+//                                               u01(z, w) -- cos for even c, sin for odd c
+constexpr uint32_t kTagBoot = 0x42540000u;
+constexpr uint32_t kTagRegion = 0x52000000u;
+constexpr int kCompactThreads = 256;
+
+// bytes of dynamic shared memory of the radius kernel: Linv and the delta columns, then one flag per
+// survivor
+size_t boot_smem(int d, int nlive)
+{
+    return adapt_smem(d) + (size_t)nlive;
+}
+
+// the exclusive prefix of flag f among the threads of the block and the block's total (every thread
+// of the block calls it; wsum: shared, one int per warp)
+__device__ __forceinline__ int block_prefix(bool f, int *wsum, int &total)
+{
+    const unsigned bal = __ballot_sync(kFull, f);
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    if (lane == 0) wsum[wid] = __popc(bal);
+    __syncthreads();
+    int pre = __popc(bal & ((1u << lane) - 1u));
+    total = 0;
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) {
+        if (w < wid) pre += wsum[w];
+        total += wsum[w];
+    }
+    __syncthreads();
+    return pre;
+}
+
+// rad2[r] = 0 for the runs taking part in the round, before the bootstraps take their maximum
+__global__ void region_clear_kernel(const LiveArgs a, double *rad2)
+{
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r < a.n_runs && a.kk[r] > 0) rad2[r] = 0.0;
+}
+
+// One block per (bootstrap b, run r) with kk[r] > 0: the survivors drawn with replacement (n draws)
+// are the selected ones; rho2_b = max over the survivors never drawn of min over the selected ones
+// of D (0 when every survivor was drawn), merged into rad2[r] by an integer atomicMax of its bits
+// (non-negative doubles order as their bit patterns): exact, whatever the order of the blocks.
+__global__ void __launch_bounds__(kAdaptThreads) region_radius_kernel(const LiveArgs a, const double *chol_all,
+                                                                      const Wrap4 wr, double *rad2)
+{
+    const int b = blockIdx.x, r = blockIdx.y, d = a.d;
+    const int64_t kk = a.kk[r];
+    if (kk <= 0) return;
+    extern __shared__ double smem[];
+    __shared__ double wmax[kAdaptThreads / 32];
+    double *Linv = smem, *dl = smem + d * (d + 1) / 2 + threadIdx.x;
+    uint8_t *chosen = (uint8_t *)(smem + d * (d + 1) / 2 + kAdaptThreads * d);
+    const int n = a.nlive - (int)kk;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) chosen[i] = 0;
+    form_linv(chol_all + (size_t)r * d * d, d, Linv);  // (ends with a barrier)
+    const uint64_t seed = a.seeds[r];
+    for (int q = threadIdx.x; 4 * q < n; q += blockDim.x) {
+        const U4 w = draw_seed(seed, a.round, kTagBoot + (uint32_t)b, (uint32_t)q);
+        const uint32_t words[4] = {w.x, w.y, w.z, w.w};
+        for (int t = 0; t < 4 && 4 * q + t < n; ++t) chosen[__umulhi(words[t], (uint32_t)n)] = 1;
+    }
+    __syncthreads();
+    const int64_t *rows = a.order + (size_t)r * a.nlive + kk;
+    const double *u = a.u_live + (size_t)r * a.nlive * d;
+    double mx = 0.0;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        if (chosen[i]) continue;
+        const double *ui = u + (size_t)rows[i] * d;
+        double mn = INFINITY;
+        for (int j = 0; j < n; ++j)
+            if (chosen[j]) mn = fmin(mn, whitened_dist2(ui, u + (size_t)rows[j] * d, d, Linv, dl, wr));
+        mx = fmax(mx, mn);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(kFull, mx, o));
+    if ((threadIdx.x & 31) == 0) wmax[threadIdx.x >> 5] = mx;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double m = wmax[0];
+        for (int i = 1; i < (int)(blockDim.x >> 5); ++i) m = fmax(m, wmax[i]);
+        atomicMax((unsigned long long *)(rad2 + r), (unsigned long long)__double_as_longlong(m));
+    }
+}
+
+// Block (x, r), thread t: candidate slot s = x blockDim.x + t < ns of run r (its slots are the rows
+// slot_base[r] .. slot_base[r + 1] - 1 of stage / flag).  Survivor i and a point y uniform in the unit
+// ball (z / |z| v^(1/d), z Gaussian); delta = (rho v^(1/d) / |z|) L z; rejected where a circular
+// |delta_c| > 1/2 (each ball is then its nearest-image ball on the torus); x = u_i + delta, a circular
+// coordinate wrapped as the slice candidates are, a non-circular one outside [0, 1) rejected; rejected
+// where a survivor j < i has D(x, u_j) <= rho2[r] (x belongs to the first ball that holds it).  flag =
+// accepted, count[r] += the run's accepted slots.
+__global__ void __launch_bounds__(kAdaptThreads) region_draw_kernel(const LiveArgs a, const double *chol_all,
+                                                                    const Wrap4 wr, const double *rad2,
+                                                                    uint32_t batch, const int32_t *slot_base,
+                                                                    double *stage, uint8_t *flag, int32_t *count)
+{
+    const int r = blockIdx.y, d = a.d, T = blockDim.x;
+    const int64_t kk = a.kk[r];
+    const int s0 = slot_base[r], ns = slot_base[r + 1] - s0;
+    if (kk <= 0 || (int)(blockIdx.x * blockDim.x) >= ns) return;  // the whole block
+    extern __shared__ double smem[];
+    double *Linv = smem, *dl = smem + d * (d + 1) / 2 + threadIdx.x;
+    const double *L = chol_all + (size_t)r * d * d;
+    form_linv(L, d, Linv);
+    const int n = a.nlive - (int)kk, s = blockIdx.x * blockDim.x + threadIdx.x;
+    bool ok = s < ns;
+    if (ok) {
+        const int64_t *rows = a.order + (size_t)r * a.nlive + kk;
+        const double *u = a.u_live + (size_t)r * a.nlive * d;
+        const uint64_t seed = a.seeds[r];
+        const uint32_t tag = kTagRegion + (batch << 8);
+        const U4 q0 = draw_seed(seed, a.round, tag, (uint32_t)s);
+        const int i = (int)__umulhi(q0.x, (uint32_t)n);
+        const double v = u01(q0.z, q0.w);
+        double n2 = 0.0;
+        for (int c = 0; c < d; ++c) {
+            const U4 q = draw_seed(seed, a.round, tag + 1u + (uint32_t)(c >> 1), (uint32_t)s);
+            const double rad = sqrt(-2.0 * log(u01(q.x, q.y))), ang = 6.283185307179586 * u01(q.z, q.w);
+            const double z = (c & 1) ? rad * sin(ang) : rad * cos(ang);
+            dl[c * T] = z;
+            n2 = n2 + z * z;
+        }
+        const double scale = sqrt(rad2[r]) * (pow(v, 1.0 / d) / sqrt(n2));
+        const double *ui = u + (size_t)rows[i] * d;
+        double *x = stage + (size_t)(s0 + s) * d;
+        for (int c = 0; c < d && ok; ++c) {
+            double acc = 0.0;
+            for (int l = 0; l <= c; ++l) acc = acc + L[(size_t)c * d + l] * dl[l * T];
+            const double dc = scale * acc, p = ui[c] + dc;
+            if (circular(wr, c)) {
+                ok = fabs(dc) <= 0.5;
+                x[c] = wrap_unit(p);
+            } else {
+                ok = p >= 0.0 && p < 1.0;
+                x[c] = p;
+            }
+        }
+        const double lim = rad2[r];
+        for (int j = 0; j < i && ok; ++j)
+            if (whitened_dist2(x, u + (size_t)rows[j] * d, d, Linv, dl, wr) <= lim) ok = false;
+    }
+    if (s < ns) flag[s0 + s] = ok ? 1 : 0;
+    const int acc = __syncthreads_count(ok);
+    if (threadIdx.x == 0 && acc) atomicAdd(count + r, acc);
+}
+
+// One block per run: offs[r] = count[0] + .. + count[r - 1] (offs[R] = the total), and the accepted
+// slots of run r, in slot order, copied to the rows offs[r] .. offs[r + 1] - 1 of cand (none for a run
+// with kk[r] = 0: the draw kernel left its flags as they were)
+__global__ void __launch_bounds__(kCompactThreads) region_compact_kernel(int n_runs, int d, const int64_t *kk,
+                                                                         const int32_t *slot_base,
+                                                                         const double *stage, const uint8_t *flag,
+                                                                         const int32_t *count, int32_t *offs,
+                                                                         double *cand)
+{
+    const int r = blockIdx.x;
+    __shared__ int wsum[kCompactThreads / 32];
+    int base = 0;
+    for (int q = 0; q < r; ++q) base += count[q];
+    if (threadIdx.x == 0) {
+        offs[r] = base;
+        if (r == n_runs - 1) offs[n_runs] = base + count[r];
+    }
+    if (kk[r] <= 0) return;
+    const int s0 = slot_base[r], ns = slot_base[r + 1] - s0;
+    for (int c0 = 0; c0 < ns; c0 += blockDim.x) {
+        const int s = c0 + threadIdx.x;
+        const bool f = s < ns && flag[s0 + s];
+        int total;
+        const int pre = block_prefix(f, wsum, total);
+        if (f)
+            for (int c = 0; c < d; ++c) cand[(size_t)(base + pre) * d + c] = stage[(size_t)(s0 + s) * d + c];
+        base += total;
+    }
+}
+
+// One block per run r with kk[r] > 0: its rows offs[r] .. offs[r + 1] - 1 with cand_ll > lmin[r], in
+// row order, fill its walkers filled[r], filled[r] + 1, .. < kk[r] (walker j of run r: the walker w of
+// the launch with run_of[w] = r, walker_of[w] = j): u, theta, lcur from the row.  filled[r] grows by
+// what was taken, above[r] = the rows above lmin[r].  sel: scratch, one int per row.
+__global__ void __launch_bounds__(kCompactThreads) region_pick_kernel(int k, int d, const int64_t *kk_all,
+                                                                      const double *lmin, const int32_t *offs,
+                                                                      const double *cand, const double *cand_th,
+                                                                      const double *cand_ll, int32_t *sel,
+                                                                      const int32_t *run_of, const int32_t *walker_of,
+                                                                      double *u, double *theta, double *lcur,
+                                                                      int32_t *filled, int32_t *above)
+{
+    const int r = blockIdx.x;
+    const int64_t need = kk_all[r];
+    if (need <= 0) return;
+    __shared__ int wsum[kCompactThreads / 32];
+    const int o0 = offs[r], nr = offs[r + 1] - o0, f0 = filled[r];
+    const double lm = lmin[r];
+    int cnt = 0;
+    for (int c0 = 0; c0 < nr; c0 += blockDim.x) {
+        const int s = c0 + threadIdx.x;
+        const bool f = s < nr && cand_ll[o0 + s] > lm;
+        int total;
+        const int pre = block_prefix(f, wsum, total);
+        if (f) sel[o0 + cnt + pre] = o0 + s;
+        cnt += total;
+    }
+    __syncthreads();
+    for (int w = threadIdx.x; w < k; w += blockDim.x) {
+        if (run_of[w] != r) continue;
+        const int t = walker_of[w] - f0;
+        if (t < 0 || t >= cnt || walker_of[w] >= need) continue;
+        const int row = sel[o0 + t];
+        for (int c = 0; c < d; ++c) {
+            u[(size_t)w * d + c] = cand[(size_t)row * d + c];
+            theta[(size_t)w * d + c] = cand_th[(size_t)row * d + c];
+        }
+        lcur[w] = cand_ll[row];
+    }
+    if (threadIdx.x == 0) {
+        filled[r] = (int32_t)(f0 + cnt < need ? f0 + cnt : need);
+        above[r] = cnt;
+    }
+}
+
 int sfail(const std::string &m)
 {
     g_slice_error = m;
@@ -719,17 +951,43 @@ int adapt_args(const rvl_slice_runs *runs, const rvl_slice_live *l, const uint32
     return RVL_OK;
 }
 
-// lets `kernel` take adapt_smem(d) bytes of dynamic shared memory (up to 197 KB at d = 128)
+// lets `kernel` take `smem` bytes of dynamic shared memory
 template <class K>
-int allow_smem(K kernel, int d)
+int allow_bytes(K kernel, size_t smem)
 {
-    const size_t smem = adapt_smem(d);
     if (smem <= 48 * 1024) return RVL_OK;
     const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) {
         g_slice_error = cudaGetErrorString(e);
         return RVL_ECUDA;
     }
+    return RVL_OK;
+}
+
+// lets `kernel` take adapt_smem(d) bytes of dynamic shared memory (up to 197 KB at d = 128)
+template <class K>
+int allow_smem(K kernel, int d)
+{
+    return allow_bytes(kernel, adapt_smem(d));
+}
+
+// the common checks of the region entry points: runs, live and their sizes, the mask, seeds / chol /
+// u_live / order / kk of the runs and live points
+int region_args(const rvl_region_args *g, const rvl_slice_runs *runs, const rvl_slice_live *l,
+                const uint32_t *wrap_bits, LiveArgs &a, Wrap4 &wr)
+{
+    if (!g) return sfail("region is NULL");
+    if (!runs) return sfail("runs is NULL");
+    if (!l) return sfail("live is NULL");
+    if (runs->n_runs < 1 || l->nlive < 3 || l->d <= 0 || l->d > kMaxDim)
+        return sfail("bad sizes (n_runs >= 1, nlive >= 3, 0 < d <= 128)");
+    if (!runs->seeds || !runs->chol || !l->u_live || !l->order || !l->kk)
+        return sfail("runs->seeds, runs->chol, live->u_live, live->order and live->kk must be set");
+    bool any = false;
+    if (const int rc = read_wrap(wrap_bits, l->d, wr.w, any)) return rc;
+    a.n_runs = runs->n_runs; a.nlive = l->nlive; a.d = l->d; a.round = l->round;
+    a.seeds = (const uint64_t *)runs->seeds; a.u_live = (double *)l->u_live;
+    a.order = (const int64_t *)l->order; a.kk = (const int64_t *)l->kk;
     return RVL_OK;
 }
 
@@ -831,6 +1089,71 @@ int rvl_slice_runs_travel(const rvl_slice_args *s, const rvl_slice_runs *runs, c
     runs_travel_kernel<<<a.n_runs, kAdaptThreads, adapt_smem(a.d), (cudaStream_t)stream>>>(
         a, s->k, (const int32_t *)runs->run_of, (const int64_t *)live->start, (const double *)s->u,
         (const double *)runs->chol, wr, rad2, far);
+    return launched();
+}
+
+int rvl_region_runs_radius(const rvl_region_args *g, const rvl_slice_runs *runs, const rvl_slice_live *live,
+                           const uint32_t wrap_bits[4], void *stream)
+{
+    LiveArgs a{};
+    Wrap4 wr{};
+    if (const int rc = region_args(g, runs, live, wrap_bits, a, wr)) return rc;
+    if (g->num_bootstraps < 1 || g->num_bootstraps > 65536) return sfail("num_bootstraps must be in [1, 65536]");
+    if (!g->rad2) return sfail("region->rad2 must be set");
+    const size_t smem = boot_smem(a.d, a.nlive);
+    if (smem > 227 * 1024) return sfail("nlive too large: the bootstrap's flags do not fit in shared memory");
+    if (const int rc = allow_bytes(region_radius_kernel, smem)) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    double *rad2 = (double *)g->rad2;
+    region_clear_kernel<<<(unsigned)((a.n_runs + 127) / 128), 128, 0, st>>>(a, rad2);
+    region_radius_kernel<<<dim3((unsigned)g->num_bootstraps, (unsigned)a.n_runs), kAdaptThreads, smem, st>>>(
+        a, (const double *)runs->chol, wr, rad2);
+    return launched();
+}
+
+int rvl_region_runs_draw(const rvl_region_args *g, const rvl_slice_runs *runs, const rvl_slice_live *live,
+                         const uint32_t wrap_bits[4], void *stream)
+{
+    LiveArgs a{};
+    Wrap4 wr{};
+    if (const int rc = region_args(g, runs, live, wrap_bits, a, wr)) return rc;
+    if (g->batch > 0xFFFFu) return sfail("region->batch must be below 65536");
+    if (g->max_slots < 0) return sfail("region->max_slots must be >= 0");
+    if (!g->rad2 || !g->slot_base || !g->stage || !g->flag || !g->count || !g->offs || !g->cand)
+        return sfail("draw: region->rad2, slot_base, stage, flag, count, offs and cand must be set");
+    if (const int rc = allow_smem(region_draw_kernel, a.d)) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    int32_t *count = (int32_t *)g->count;
+    const int32_t *slot_base = (const int32_t *)g->slot_base;
+    if (cudaMemsetAsync(count, 0, sizeof(int32_t) * a.n_runs, st) != cudaSuccess) return launched();
+    if (g->max_slots > 0)
+        region_draw_kernel<<<dim3((unsigned)((g->max_slots + kAdaptThreads - 1) / kAdaptThreads), (unsigned)a.n_runs),
+                             kAdaptThreads, adapt_smem(a.d), st>>>(a, (const double *)runs->chol, wr,
+                                                                   (const double *)g->rad2, g->batch, slot_base,
+                                                                   (double *)g->stage, (uint8_t *)g->flag, count);
+    region_compact_kernel<<<a.n_runs, kCompactThreads, 0, st>>>(a.n_runs, a.d, a.kk, slot_base, (const double *)g->stage,
+                                                                (const uint8_t *)g->flag, count,
+                                                                (int32_t *)g->offs, (double *)g->cand);
+    return launched();
+}
+
+int rvl_region_runs_pick(const rvl_region_args *g, const rvl_slice_args *s, const rvl_slice_runs *runs,
+                         const rvl_slice_live *live, void *stream)
+{
+    if (!g) return sfail("region is NULL");
+    if (!s) return sfail("args is NULL");
+    if (!runs) return sfail("runs is NULL");
+    if (!live) return sfail("live is NULL");
+    if (runs->n_runs < 1 || s->k <= 0 || s->d <= 0 || s->d > kMaxDim || s->d != live->d)
+        return sfail("bad sizes (n_runs >= 1, args->k > 0, 0 < d <= 128, args->d == live->d)");
+    if (!g->offs || !g->cand || !g->cand_th || !g->cand_ll || !g->sel || !g->filled || !g->above ||
+        !s->u || !s->theta || !s->lcur || !runs->run_of || !runs->walker_of || !runs->lmin || !live->kk)
+        return sfail("pick: a device address is missing");
+    region_pick_kernel<<<runs->n_runs, kCompactThreads, 0, (cudaStream_t)stream>>>(
+        s->k, s->d, (const int64_t *)live->kk, (const double *)runs->lmin, (const int32_t *)g->offs,
+        (const double *)g->cand, (const double *)g->cand_th, (const double *)g->cand_ll, (int32_t *)g->sel,
+        (const int32_t *)runs->run_of, (const int32_t *)runs->walker_of, (double *)s->u, (double *)s->theta,
+        (double *)s->lcur, (int32_t *)g->filled, (int32_t *)g->above);
     return launched();
 }
 

@@ -18,6 +18,10 @@ more moves while most walkers end within the live set's largest nearest-neighbou
 started, fewer when most leave it, measured in the moves' whitened metric by
 ``rvl_slice_runs_radius`` / ``_travel`` (DESIGN.md section 9.1).
 
+``nested_sample_ensemble(method='mlfriends')`` (opt-in) fills each round's walkers by MLFriends region
+sampling instead of slice moves: independent draws from the union of balls around the survivors
+(``rvl_region_runs_*``, DESIGN.md section 9.1).
+
 Same algorithm (SURVEY.md 8f row 1; the scheme of PolyChord / UltraNest's step samplers that the
 reference configures at evidence/ultranest/__init__.py:175): per round the k worst live points are
 retired with the shrinkage 1/n for n = nlive, nlive-1, ..; k walkers started from surviving live
@@ -599,9 +603,9 @@ class _NativeSliceRuns(_NativeSlice):
         self._check(self.lib.rvl_slice_runs_init(self._runs, self._live, self._stream()), "rvl_slice_runs_init")
         return self.u_live
 
-    def setup_round(self, th_live, l_live, order, kk, lmin, run_of, walker_of, round_no):
+    def setup_round(self, th_live, l_live, order, kk, lmin, run_of, walker_of, round_no, starts=True):
         """Whitening of every run and the starts of the round's walkers (the layout run_of /
-        walker_of, int32 device tensors of the reserved length)."""
+        walker_of, int32 device tensors of the reserved length); ``starts=False``: the whitening only."""
         lv, rn = self.live, self.runs
         lv.th_live, lv.l_live, lv.order, lv.kk = (th_live.data_ptr(), l_live.data_ptr(), order.data_ptr(),
                                                   kk.data_ptr())
@@ -609,8 +613,9 @@ class _NativeSliceRuns(_NativeSlice):
         rn.lmin, rn.run_of, rn.walker_of = lmin.data_ptr(), run_of.data_ptr(), walker_of.data_ptr()
         self._check(self.lib.rvl_slice_runs_whiten(self._runs, self._live, self.wrap_bits, self._stream()),
                     "rvl_slice_runs_whiten")
-        self._check(self.lib.rvl_slice_runs_starts(self._byref, self._runs, self._live, self._stream()),
-                    "rvl_slice_runs_starts")
+        if starts:
+            self._check(self.lib.rvl_slice_runs_starts(self._byref, self._runs, self._live, self._stream()),
+                        "rvl_slice_runs_starts")
 
     def moves_prefix(self, fused, lmin, ks):
         """Adaptive moves of a round laid out by ``_adaptive_layout``: move j launches the first ks[j]
@@ -633,9 +638,116 @@ class _NativeSliceRuns(_NativeSlice):
                     "rvl_slice_runs_travel")
 
 
+def _region_batch(need, eff, ndraw_max):
+    """The candidate slots of each run in a batch of MLFriends draws (int64 arrays over runs):
+    clamp(ceil(1.5 need / eff), need, ndraw_max) for a run that still needs walkers, 0 otherwise.
+    ``eff``: the run's accepted-above-L* per geometric draw over its previous round (1 at the start)."""
+    need = np.asarray(need, dtype=np.int64)
+    eff = np.asarray(eff, dtype=np.float64)
+    want = np.ceil(1.5 * need / eff).astype(np.int64)
+    c = np.minimum(np.maximum(want, need), int(ndraw_max))
+    return np.where(need > 0, c, 0)
+
+
+class _RegionRuns:
+    """
+    MLFriends region sampling of an ensemble's walkers through ``rvl_region_runs_radius`` / ``_draw``
+    / ``_pick`` (csrc/rvslice.cu).  A round: the bootstrapped radius of every run, then batches of
+    draw -> one likelihood launch over the accepted rows -> pick, until every run's walkers are
+    filled.  Each batch reads back the compacted row offsets and the filled counts.  A run's batch
+    sizes depend on its own need and efficiency alone (``_region_batch``), so its draws do not depend
+    on the other runs.
+    """
+
+    def __init__(self, torch, ns, num_bootstraps, ndraw_max):
+        import ctypes
+        from . import _abi
+        self.torch, self.ns, self.ndraw_max = torch, ns, int(ndraw_max)
+        R, dev = ns.n_runs, ns.dev
+        i32 = torch.int32
+        self.rad2 = torch.zeros(R, dtype=torch.float64, device=dev)
+        self.slot_base = torch.zeros(R + 1, dtype=i32, device=dev)
+        self.count = torch.zeros(R, dtype=i32, device=dev)
+        self.offs = torch.zeros(R + 1, dtype=i32, device=dev)
+        self.fill_above = torch.zeros((2, R), dtype=i32, device=dev)  # filled, above: one read-back
+        self.up = torch.zeros(R + 1, dtype=i32).pin_memory()
+        self.args = _abi.rvl_region_args(num_bootstraps=int(num_bootstraps), rad2=self.rad2.data_ptr(),
+                                         slot_base=self.slot_base.data_ptr(), count=self.count.data_ptr(),
+                                         offs=self.offs.data_ptr(), filled=self.fill_above[0].data_ptr(),
+                                         above=self.fill_above[1].data_ptr())
+        self._byref = ctypes.byref(self.args)
+        self.eff = np.ones(R)
+        self.draws = np.zeros(R, dtype=np.int64)
+        self.cap = 0
+
+    def _reserve(self, S):
+        torch, ns = self.torch, self.ns
+        if S > self.cap:
+            S = max(S, 2 * self.cap)
+            f64, dev, d = torch.float64, ns.dev, ns.d
+            self.stage, self.cand, self.th = (torch.zeros((S, d), dtype=f64, device=dev) for _ in range(3))
+            self.ll = torch.zeros(S, dtype=f64, device=dev)
+            self.flag = torch.zeros(S, dtype=torch.uint8, device=dev)
+            self.sel = torch.zeros(S, dtype=torch.int32, device=dev)
+            a = self.args
+            a.stage, a.cand, a.cand_th, a.cand_ll = (self.stage.data_ptr(), self.cand.data_ptr(), self.th.data_ptr(),
+                                                     self.ll.data_ptr())
+            a.flag, a.sel = self.flag.data_ptr(), self.sel.data_ptr()
+            self.cap = S
+
+    def fill(self, fused, counts, max_calls, ncall):
+        """Fill the walkers of the round (counts[r] for run r; ns.setup_round(starts=False) done):
+        ns.u / theta / lcur.  Adds each run's evaluated rows to ncall (in place) and its geometric
+        draws to ``draws``; updates each run's efficiency."""
+        ns, torch = self.ns, self.torch
+        stream = ns._stream()
+        ns._check(ns.lib.rvl_region_runs_radius(self._byref, ns._runs, ns._live, ns.wrap_bits, stream),
+                  "rvl_region_runs_radius")
+        counts = np.asarray(counts, dtype=np.int64)
+        self.fill_above.zero_()
+        filled = np.zeros_like(counts)
+        above, drawn = np.zeros_like(counts), np.zeros_like(counts)
+        inplace = _NativeSlice._writes_in_place(fused)
+        batch = 0
+        while (filled < counts).any():
+            if batch > 0xFFFF:
+                raise RuntimeError("nested_sample_ensemble: more than 65536 batches of region draws in a round")
+            c = _region_batch(counts - filled, self.eff, self.ndraw_max)
+            base = np.concatenate([[0], np.cumsum(c)])
+            self._reserve(int(base[-1]))
+            self.up[:] = torch.from_numpy(base.astype(np.int32))
+            self.slot_base.copy_(self.up, non_blocking=True)
+            self.args.batch, self.args.max_slots = batch, int(c.max())
+            ns._check(ns.lib.rvl_region_runs_draw(self._byref, ns._runs, ns._live, ns.wrap_bits, stream),
+                      "rvl_region_runs_draw")
+            offs = self.offs.cpu().numpy().astype(np.int64)  # read-back 1: the compacted rows
+            total = int(offs[-1])
+            if total:
+                if inplace:
+                    fused(self.cand[:total], theta=self.th[:total], lnl=self.ll[:total])
+                else:
+                    th, ll = fused(self.cand[:total])
+                    self.th[:total].copy_(th)
+                    self.ll[:total].copy_(ll)
+            ns._check(ns.lib.rvl_region_runs_pick(self._byref, ns._byref, ns._runs, ns._live, stream),
+                      "rvl_region_runs_pick")
+            fa = self.fill_above.cpu().numpy()  # read-back 2: the filled counts
+            filled = fa[0].astype(np.int64)
+            above += fa[1]
+            drawn += c
+            ncall += np.diff(offs)
+            self.draws += c
+            batch += 1
+            if (ncall > max_calls).any() or (self.draws > max_calls).any():
+                raise RuntimeError("nested_sample_ensemble: max_calls exceeded")
+        busy = counts > 0
+        self.eff[busy] = np.maximum(above[busy] / drawn[busy], 1.0 / self.ndraw_max)
+
+
 def nested_sample_ensemble(fused, ndim, seeds, nlive=400, dlogz=0.5, frac_remain=0.01, nsteps=None,
                            wrapped=None, device="cuda", native_m=8, native_rounds=3, native_out=8,
-                           num_bootstraps=30, max_calls=2_000_000_000, adaptive_nsteps=None, max_nsteps=None):
+                           num_bootstraps=30, max_calls=2_000_000_000, adaptive_nsteps=None, max_nsteps=None,
+                           method="slice", ndraw_max=65536):
     """
     R = len(seeds) independent runs of ``nested_sample_device`` (native kernels, batch_fraction 0.2)
     on one likelihood, advanced in lockstep: every bookkeeping launch and every likelihood launch
@@ -661,8 +773,23 @@ def nested_sample_ensemble(fused, ndim, seeds, nlive=400, dlogz=0.5, frac_remain
     points and walkers alone.  A round lays the walkers out with runs sorted by their count,
     descending (``_adaptive_layout``), so that move j launches only the walkers still moving, a
     prefix.  The far walkers' counts ride on the round's read-back as a fifth column.
+
+    ``method='mlfriends'`` (opt-in; the default 'slice' is the slice sampler above): the walkers of a
+    round are filled by MLFriends region sampling (``_RegionRuns``) instead of slice moves -- each
+    replacement an independent draw from the prior restricted to the union of balls of radius rho
+    around the run's survivors, in the whitened metric of ``rvl_slice_runs_whiten``, rho from
+    ``num_bootstraps`` bootstraps of the nearest-neighbour distances, and accepted above L*.  That
+    region follows several modes at once.  Retirement, termination and results are shared with the
+    slice path.  A run draws at most ``ndraw_max`` candidates per batch; ``ncall`` counts the
+    evaluated rows (the candidates inside the region), ``region_draws`` every geometric draw, and
+    ``max_calls`` bounds both.  ``nsteps`` and the slice settings are not used;
+    ``adaptive_nsteps`` is a ValueError with it.
     """
     import torch
+    if method not in ("slice", "mlfriends"):
+        raise ValueError(f"method: {method!r}; 'slice' or 'mlfriends'")
+    if method == "mlfriends" and adaptive_nsteps is not None:
+        raise ValueError("adaptive_nsteps applies to method='slice' only, not 'mlfriends'")
     seeds = _ensemble_seeds(seeds)
     wmask = wrap_mask(wrapped, ndim)
     dev = torch.device(device)
@@ -706,6 +833,7 @@ def nested_sample_ensemble(fused, ndim, seeds, nlive=400, dlogz=0.5, frac_remain
         history = [[] for _ in range(R)]
         rad2 = torch.zeros(R, dtype=f64, device=dev)
         far = torch.zeros(R, dtype=torch.int32, device=dev)
+    region = _RegionRuns(torch, ns, num_bootstraps, ndraw_max) if method == "mlfriends" else None
     while active.any():
         act = np.flatnonzero(active)
         kk = np.minimum(kk, nlive - 2)
@@ -750,8 +878,10 @@ def nested_sample_ensemble(fused, ndim, seeds, nlive=400, dlogz=0.5, frac_remain
                             root_live[r, worst][None], birth_live[r, worst][None]))
         ns.reserve(K)
         lmin = l_sorted.gather(1, (kk_dev - 1).clamp(min=0)[:, None]).reshape(R)
-        ns.setup_round(th_live, l_live, order, kk_dev, lmin, run_t, walker_t, round_no)
-        if adaptive:
+        ns.setup_round(th_live, l_live, order, kk_dev, lmin, run_t, walker_t, round_no, starts=region is None)
+        if region is not None:
+            region.fill(fused, counts, max_calls, ncall)
+        elif adaptive:
             ns.radius(rad2)
             ns.move = _move_base(round_no, cap)
             ns.moves_prefix(fused, lmin, ks)
@@ -795,13 +925,15 @@ def nested_sample_ensemble(fused, ndim, seeds, nlive=400, dlogz=0.5, frac_remain
                                 root_live[r, o][None], birth_live[r, o][None]))
                 active[r] = False
     return _ensemble_results(records, logz.cpu().numpy(), ns.stats.cpu().numpy(), seeds, ncall, niter,
-                             nlive, ndim, wmask, num_bootstraps, history if adaptive else None)
+                             nlive, ndim, wmask, num_bootstraps, history if adaptive else None,
+                             region_draws=None if region is None else region.draws)
 
 
 def _ensemble_results(records, logz, stats, seeds, ncall, niter, nlive, ndim, wmask, num_bootstraps,
-                      history=None):
+                      history=None, region_draws=None):
     """One NestedResult per run from the retirement records of an ensemble (host numpy; each run's
-    arrays in the order its points died, as nested_sample_device keeps them)."""
+    arrays in the order its points died, as nested_sample_device keeps them).  ``region_draws``: the
+    geometric draws of each run of an MLFriends ensemble (its results then say so)."""
     import torch
     host = [torch.cat([rec[1 + j].reshape((-1, ndim) if j == 0 else (-1,)) for rec in records]).cpu().numpy()
             for j in range(5)]
@@ -835,4 +967,7 @@ def _ensemble_results(records, logz, stats, seeds, ncall, niter, nlive, ndim, wm
                                 wrapped=wmask))
         if history is not None:
             out[-1]["nsteps_history"] = history[r]
+        if region_draws is not None:
+            out[-1]["method"] = "mlfriends-device-ensemble"
+            out[-1]["region_draws"] = int(region_draws[r])
     return out

@@ -12,16 +12,21 @@ post-processing and pickles stay compatible.  What changes is the hot loop: the 
 Extra ``ultrasettings`` keys (the "config switch"):
     'vectorized' (True), 'ndraw_min' (4096), 'ndraw_max' (65536), 'seed' (None),
     'stepsampler' ('region-slice' like the reference | 'population-slice' | 'none'),
-    'sampler' ('auto' | 'ultranest' | 'builtin'), 'builtin_method' ('slice' | 'slice-device' | 'ellipsoid'),
-    'builtin_wrap' (False: the built-in slice samplers take the wrapped parameters -- the ones UltraNest
-    gets as ``wrapped_params`` -- as circular coordinates; 'ellipsoid' rejects it),
+    'sampler' ('auto' | 'ultranest' | 'builtin'),
+    'builtin_method' ('slice' | 'slice-device' | 'ellipsoid' | 'mlfriends-device': MLFriends region
+    sampling on the device, ``sampler_dev.nested_sample_ensemble(method='mlfriends')``, run as an
+    ensemble of one seed, at most 'ndraw_max' candidates per batch),
+    'builtin_wrap' (False: the built-in slice samplers and 'mlfriends-device' take the wrapped
+    parameters -- the ones UltraNest gets as ``wrapped_params`` -- as circular coordinates; 'ellipsoid'
+    rejects it),
     'builtin_adaptive_nsteps' (False | 'move-distance': the device sampler adapts each run's number of
     moves per round, ``sampler_dev.nested_sample_device(adaptive_nsteps=...)``; 'slice-device' and
     ``run_ensemble`` only, 'slice' and 'ellipsoid' reject it),
     'postprocess' (False), 'plot' (False)
 
-``run_ensemble`` runs several seeded runs of the built-in device sampler through shared launches and
-writes each as ``run()`` would (one run directory, pickle and ``weighted_post.txt`` per run).
+``run_ensemble`` runs several seeded runs of the built-in device sampler ('mlfriends-device' or, for
+any other 'builtin_method', the slice sampler) through shared launches and writes each as ``run()``
+would (one run directory, pickle and ``weighted_post.txt`` per run).
 
 UltraNest is a third-party package that is not part of the reference repository (SURVEY.md 8c).
 When it is importable it is used; otherwise -- or with ``'sampler': 'builtin'`` -- the seeded
@@ -146,7 +151,18 @@ def run(model, rundict, priordict, ultrasettings=None):
         if adaptive is not None and settings["builtin_method"] != "slice-device":
             raise ValueError(f"'builtin_adaptive_nsteps': {adaptive!r} needs 'builtin_method': 'slice-device', "
                              f"not {settings['builtin_method']!r}")
-        if settings["builtin_method"] == "slice-device":
+        if settings["builtin_method"] == "mlfriends-device":
+            # MLFriends region sampling on the likelihood's device: an ensemble of one seed
+            from .sampler_dev import nested_sample_ensemble
+            if not hasattr(model, "transform_loglike_device"):
+                raise ValueError("'builtin_method': 'mlfriends-device' needs the device model")
+            res = nested_sample_ensemble(model.transform_loglike_device, ndim,
+                                         [0 if settings["seed"] is None else settings["seed"]],
+                                         nlive=settings["nlive"], dlogz=settings["dlogz"],
+                                         frac_remain=settings["frac_remain"], wrapped=builtin_wrapped,
+                                         device=_torch_device(model), num_bootstraps=settings["num_bootstraps"],
+                                         method="mlfriends", ndraw_max=settings["ndraw_max"])[0]
+        elif settings["builtin_method"] == "slice-device":
             # the whole run on the likelihood's device (evidence_b200.sampler_dev)
             from .sampler_dev import nested_sample_device
             if not hasattr(model, "transform_loglike_device"):
@@ -169,6 +185,9 @@ def run(model, rundict, priordict, ultrasettings=None):
         # file, and the implementation named beside it
         name = "UltraNest"
         impl = f"evidence_b200.sampler ({settings['builtin_method']}); ultranest not used"
+        if settings["builtin_method"] == "mlfriends-device":
+            impl = (f"evidence_b200.sampler_dev (mlfriends-device: MLFriends region sampling, "
+                    f"{settings['num_bootstraps']} bootstraps); ultranest not used")
         if builtin_wrapped is not None:
             impl += "; wrapped: " + (", ".join(p for p, w in zip(parnames, wrapped) if w) or "none")
         if adaptive is not None:
@@ -245,6 +264,8 @@ def run_ensemble(model, rundict, priordict, ultrasettings=None, nruns=4, seeds=N
     'seed', 0 when None) sets nruns.  Every output's runtime, walltime, ``device_counters`` and
     ``evals_per_second`` (all runs' evaluations over the wall time) are those of the whole ensemble,
     which is what the GPU did; ``nlike`` is the run's own count.  Settings as for ``run()``;
+    'builtin_method': 'mlfriends-device' runs MLFriends region sampling
+    (``nested_sample_ensemble(method='mlfriends')``), any other value the slice sampler;
     'builtin_wrap' and 'builtin_adaptive_nsteps' are honoured, and 'postprocess' runs the reference's
     post-processing on each run's own directory (``<save_dir>/<file_root>``), as ``run()`` does.
     """
@@ -264,6 +285,11 @@ def run_ensemble(model, rundict, priordict, ultrasettings=None, nruns=4, seeds=N
     wrapped = np.array([("omega" in p) or ("ml0" in p) for p in parnames], dtype=bool)
     builtin_wrapped = wrapped if base["builtin_wrap"] else None
     adaptive = _adaptive_setting(base)
+    mlfriends = base["builtin_method"] == "mlfriends-device"
+    if adaptive is not None and mlfriends:
+        raise ValueError(f"'builtin_adaptive_nsteps': {adaptive!r} needs the slice sampler, not "
+                         "'builtin_method': 'mlfriends-device'")
+    region = dict(method="mlfriends", ndraw_max=base["ndraw_max"]) if mlfriends else {}
     model.set_priors(priordict)
     ti = time.process_time()
     t_wall = time.perf_counter()
@@ -271,7 +297,7 @@ def run_ensemble(model, rundict, priordict, ultrasettings=None, nruns=4, seeds=N
                                      dlogz=base["dlogz"], frac_remain=base["frac_remain"],
                                      nsteps=base["nsteps"], wrapped=builtin_wrapped,
                                      device=_torch_device(model), num_bootstraps=base["num_bootstraps"],
-                                     adaptive_nsteps=adaptive)
+                                     adaptive_nsteps=adaptive, **region)
     tf = time.process_time()
     t_wall = time.perf_counter() - t_wall
     if size > 1:
@@ -284,7 +310,8 @@ def run_ensemble(model, rundict, priordict, ultrasettings=None, nruns=4, seeds=N
         settings = set_ultrasettings(rd, ultrasettings, ndim, 0, isodate, parnames)
         os.makedirs(settings["log_dir"], exist_ok=True)
         write_weighted_post(settings["log_dir"], parnames, res)
-        impl = (f"evidence_b200.sampler_dev ensemble (slice-device): run {i} of {len(seeds)}, seed {seed}; "
+        kind = "mlfriends-device: MLFriends region sampling" if mlfriends else "slice-device"
+        impl = (f"evidence_b200.sampler_dev ensemble ({kind}): run {i} of {len(seeds)}, seed {seed}; "
                 "ultranest not used")
         if builtin_wrapped is not None:
             impl += "; wrapped: " + (", ".join(p for p, w in zip(parnames, wrapped) if w) or "none")

@@ -477,6 +477,57 @@ int rvl_slice_runs_radius(const rvl_slice_runs *runs, const rvl_slice_live *live
                           double *rad2, void *stream);
 int rvl_slice_runs_travel(const rvl_slice_args *args, const rvl_slice_runs *runs, const rvl_slice_live *live,
                           const uint32_t wrap_bits[4], const double *rad2, int32_t *far, void *stream);
+
+/* MLFriends region sampling for the runs of an ensemble (sampler_dev: method='mlfriends'): the
+ * replacement points of a round are independent draws from the prior restricted to the union of the
+ * balls D(x, u_i) <= rho2[r] around run r's survivors u_i = u_live[r][order[r][kk[r] + i]], i < n =
+ * nlive - kk[r], D the distance of rvl_slice_runs_radius under chol[r] (rvl_slice_runs_whiten),
+ * circular coordinates of wrap_bits (may be NULL) to the nearest image.  Random numbers: Philox4x32-10
+ * under seeds[r] with live->round as the first counter word; csrc/rvslice.cu lists the counters.  Each
+ * run's values come from its own points and seed alone, whatever R.  A run with kk[r] = 0 is skipped.
+ * One round: _radius, then batches of _draw -> the likelihood of cand rows 0 .. offs[R] - 1 (into
+ * cand_th, cand_ll) -> _pick, until every run's kk[r] walkers are filled.  All addresses are device
+ * addresses; S is the batch's number of slots, slot_base[R]. */
+typedef struct {
+    int32_t num_bootstraps; /* _radius: B >= 1                                                      */
+    uint32_t batch;         /* _draw: the batch's index inside the round (< 65536; a counter word)   */
+    int32_t max_slots;      /* _draw: the largest slot count of one run in the batch                 */
+    int32_t reserved;
+    uint64_t rad2;      /* double*        [R]        rho^2 of each run (out of _radius, in for _draw) */
+    uint64_t slot_base; /* const int32_t* [R + 1]    the slots of run r are slot_base[r] .. [r + 1] - 1 */
+    uint64_t stage;     /* double*        [S][d]     scratch: every slot's candidate                 */
+    uint64_t flag;      /* uint8_t*       [S]        scratch: 1 = accepted by the geometric test     */
+    uint64_t count;     /* int32_t*       [R]        out of _draw: accepted slots of each run        */
+    uint64_t offs;      /* int32_t*       [R + 1]    out of _draw: exclusive prefix sum of count     */
+    uint64_t cand;      /* double*        [S][d]     out of _draw: the accepted candidates, run-major */
+    uint64_t cand_th;   /* const double*  [S][d]     in for _pick: their parameters                  */
+    uint64_t cand_ll;   /* const double*  [S]        in for _pick: their lnL                         */
+    uint64_t sel;       /* int32_t*       [S]        scratch of _pick                                */
+    uint64_t filled;    /* int32_t*       [R]        in/out of _pick: walkers of each run filled     */
+    uint64_t above;     /* int32_t*       [R]        out of _pick: rows of the batch above lmin[r]   */
+} rvl_region_args;
+/*   _radius  one block per (bootstrap b < B, run r): n survivor indices drawn with replacement; rho2_b
+ *            = max over the survivors never drawn of min over the drawn ones of D (0 if none is left
+ *            out); rad2[r] = max over b, exact whatever the order of the blocks.  nlive + the
+ *            distance scratch of d must fit in 227 KB of shared memory.
+ *   _draw    slot s of run r: survivor i uniform; y uniform in the unit d-ball; delta = sqrt(rad2[r])
+ *            L y; rejected if |delta_c| > 1/2 in a circular coordinate; x = u_i + delta, circular
+ *            coordinates wrapped as rvl_slice_phase_wrapped does; rejected if another coordinate is
+ *            outside [0, 1) or if a survivor j < i has D(x, u_j) <= rad2[r].  The accepted points are
+ *            uniform on the union of the balls (each is produced through the first ball that holds
+ *            it).  They go to cand, run by run in slot order; count[r] and offs (offs[R] = the total).
+ *   _pick    walker j of run r (run_of[w] = r, walker_of[w] = j of args) with filled[r] <= j < kk[r]
+ *            takes the (j - filled[r])-th row of run r with cand_ll > lmin[r], in row order: args->u,
+ *            args->theta, args->lcur.  filled[r] += the walkers taken; above[r] = such rows.
+ *            args->d == live->d.
+ * Errors: RVL_EINVAL with a message in rvl_slice_last_error for bad sizes, a missing address, B < 1
+ * or a mask bit at or above d. */
+int rvl_region_runs_radius(const rvl_region_args *region, const rvl_slice_runs *runs, const rvl_slice_live *live,
+                           const uint32_t wrap_bits[4], void *stream);
+int rvl_region_runs_draw(const rvl_region_args *region, const rvl_slice_runs *runs, const rvl_slice_live *live,
+                         const uint32_t wrap_bits[4], void *stream);
+int rvl_region_runs_pick(const rvl_region_args *region, const rvl_slice_args *args, const rvl_slice_runs *runs,
+                         const rvl_slice_live *live, void *stream);
 const char *rvl_slice_last_error(void);
 
 #ifdef __cplusplus
