@@ -14,6 +14,7 @@ SRC_FIP = os.path.join(_HERE, "csrc", "rvfip.cu")
 SRC_ORDER = os.path.join(_HERE, "csrc", "rvorder.cu")
 SRC_SLICE = os.path.join(_HERE, "csrc", "rvslice.cu")
 DEPS = [SRC, SRC_FIP, SRC_ORDER, SRC_SLICE, os.path.join(_HERE, "csrc", "rvl_math.h"),
+        os.path.join(_HERE, "csrc", "rvl_lean.h"),
         os.path.join(_HERE, "csrc", "rvl_sintab.h"),
         os.path.join(os.path.dirname(_HERE), "include", "rvlnl.h")]
 OUT = os.path.join(_HERE, "librvlnl.so")

@@ -35,6 +35,7 @@
 #include <vector>
 
 #include "../../include/rvlnl.h"
+#include "rvl_lean.h"
 #include "rvl_math.h"
 
 namespace {
@@ -191,33 +192,18 @@ __device__ __forceinline__ int lds_u8(uint32_t addr)
     return (int)v;
 }
 
-// ---- the sin/cos table of rvl::sincos_tab (rvl_sintab.h) ---------------------------------------
-// In global memory as two arrays, the (sin, cos) hi parts and then the lo parts; every block that
-// runs the lean Newton loop copies both into its shared memory once, and the loop reads them
-// through SmemSinTab.  Two arrays rather than one of whole rows: a 16-byte load of rows with a
-// 16-byte stride spreads 32 random rows over twice the banks that a 32-byte stride would.
-__device__ const double2 g_sintab_hi[rvl::kSinTabN] = {RVL_SINTAB(RVL_SINTAB_HI_ROW)};
-__device__ const double2 g_sintab_lo[rvl::kSinTabN] = {RVL_SINTAB(RVL_SINTAB_LO_ROW)};
+// ---- the sin/cos table of rvl::sincos_tab and the path thresholds (rvl_lean.h) ------------------
+using rvl::g_sintab_hi;
+using rvl::g_sintab_lo;
+using rvl::SmemSinTab;
+using rvl::kHiTrigMax;
+using rvl::kHiTiny;
+using rvl::kHiSmall;
+using rvl::kHiMid;
+using rvl::kHiMedium;
 constexpr unsigned kSinTabHiBytes = rvl::kSinTabN * sizeof(double2);
 constexpr unsigned kSinTabBytes = 2 * kSinTabHiBytes;
 static_assert(kSinTabBytes % 128 == 0, "the epoch columns behind the table stay 128-byte aligned");
-
-struct SmemSinTab {
-    uint32_t hi;  // shared-window address of the hi rows; the lo rows follow them
-    __device__ __forceinline__ rvl::TabRow operator()(int32_t j) const
-    {
-        // (not volatile: the table does not change once it is in shared memory, so the loads
-        // may be scheduled like arithmetic)
-        rvl::TabRow t;
-        // one address for both loads (left to itself the compiler shifts, masks and adds)
-        uint32_t a;
-        asm("mad.lo.u32 %0, %1, 16, %2;" : "=r"(a) : "r"(j), "r"(hi));
-        asm("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(t.sh), "=d"(t.ch) : "r"(a));
-        asm("ld.shared.v2.f64 {%0, %1}, [%2+16384];" : "=d"(t.sl), "=d"(t.cl) : "r"(a));
-        return t;
-    }
-};
-static_assert(kSinTabHiBytes == 16384, "SmemSinTab addresses the lo rows at +16384");
 
 // huge / non-finite arguments: CUDA libdevice (Payne-Hanek), out of line and returned by value
 __device__ __noinline__ double2 sincos_slow(double x)
@@ -228,14 +214,9 @@ __device__ __noinline__ double2 sincos_slow(double x)
 }
 // high word of |x| as an integer: orders like |x| itself (positive doubles sort as integers)
 __device__ __forceinline__ int abs_hi(double x) { return __double2hiint(x) & 0x7fffffff; }
-constexpr int kHiTrigMax = 0x40F86A00;  // 1e5 = 0x40F86A0000000000: |x| < 1e5  <=>  abs_hi < this
-constexpr int kHiTiny = 0x3F500000;     // abs_hi(d) <  this  <=>  |d| <  2^-10
-constexpr int kHiSmall = 0x3FA00000;    // abs_hi(d) <  this  <=>  |d| <  2^-5
 #ifndef RVL_MEDIUM
 #define RVL_MEDIUM 1
 #endif
-constexpr int kHiMid = 0x3FC00000;      // abs_hi(d) <  this  <=>  |d| <  2^-3
-constexpr int kHiMedium = 0x3FE80000;   // abs_hi(d) <  this  <=>  |d| <  0.75
 
 template <int U>
 __device__ __forceinline__ bool any_big(const double (&E)[U])

@@ -15,6 +15,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include "../../evidence_b200/csrc/rvl_lean.h"
 #include "../../evidence_b200/csrc/rvl_math.h"
 #include "../../include/rvlnl.h"
 
@@ -31,7 +32,7 @@ inline double par_of(const rvl_param &p, const double *row) { return p.slot >= 0
 
 
 inline int abs_hi(double x) { return rvl::hi32(x) & 0x7fffffff; }
-constexpr int kHiTrigMax = 0x40F86A00, kHiTiny = 0x3F500000, kHiSmall = 0x3FA00000, kHiMid = 0x3FC00000, kHiMedium = 0x3FE80000;
+using rvl::kHiTrigMax, rvl::kHiTiny, rvl::kHiSmall, rvl::kHiMid, rvl::kHiMedium;
 
 // one planet for U chunks of 32 epochs (U*32 solves) in lock-step: mirrors solve_planet<0, U>
 void solve_planet_warp(int U, const double *const *t, const double *pc, double tol, int itmax,

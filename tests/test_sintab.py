@@ -14,6 +14,7 @@ import sys
 import numpy as np
 import pytest
 
+from _mp import sincos_args, sincos_dd, sincos_err
 from _util import ROOT, lnl_close, load_golden, oracle_model
 
 from evidence_b200.layout import compile_model
@@ -42,38 +43,6 @@ def test_committed_table_is_the_generators_output():
         assert f.read() == make_sintab.render()
 
 
-def _args():
-    rng = np.random.default_rng(7)
-    h = 2 * np.pi / 1024
-    k = rng.integers(-16000, 16000, 60000).astype(np.float64)
-    tiny = np.ldexp(1.0, -np.arange(1, 1075, 7))  # down to the smallest denormal
-    edge = 1e5 - np.ldexp(1.0, -np.arange(0, 37, 2))
-    return np.concatenate([
-        rng.uniform(-1e5, 1e5, 700000),
-        rng.uniform(-1e4, 1e4, 100000),
-        rng.uniform(-7.0, 7.0, 100000),
-        k * h,                                            # multiples of 2 pi / 1024 (= pi / 512)
-        k * h * (1 + rng.uniform(-4e-16, 4e-16, len(k))),  # ... and their neighbours
-        k * h + h / 2,                                    # halfway between two rows
-        rng.uniform(-1e-3, 1e-3, 20000),
-        tiny, -tiny, [0.0, -0.0, 5e-324, -5e-324],
-        edge, -edge,
-    ])
-
-
-def _reference(x):
-    """(sin, cos) of each x as double-doubles from 120-bit mpmath: hi correctly rounded."""
-    from mpmath.libmp import from_float, mpf_cos_sin, mpf_sub, round_nearest, to_float
-    rn = round_nearest
-    out = np.empty((len(x), 4))
-    for i, v in enumerate(x.tolist()):
-        c, s = mpf_cos_sin(from_float(v), 120, rn)
-        sh, ch = to_float(s, rnd=rn), to_float(c, rnd=rn)
-        out[i] = (sh, ch, to_float(mpf_sub(s, from_float(sh), 120, rn), rnd=rn),
-                  to_float(mpf_sub(c, from_float(ch), 120, rn), rnd=rn))
-    return out
-
-
 def _eval(fn, x):
     s = np.empty_like(x)
     c = np.empty_like(x)
@@ -82,14 +51,13 @@ def _eval(fn, x):
 
 
 def test_sincos_tab_accuracy(lib):
-    x = np.ascontiguousarray(_args())
+    x = sincos_args()
     assert len(x) >= 10**6 and np.abs(x).max() < 1e5
-    ref = _reference(x)
+    ref = sincos_dd(x)
     report = {}
     for name, fn in (("sincos_tab", lib.emul_sincos_tab), ("sincos_fast", lib.emul_sincos_fast)):
         s, c = _eval(fn, x)
-        # got - hi is exact (a few ulp apart), so the error is known to ~1e-32
-        err = np.maximum(np.abs((s - ref[:, 0]) - ref[:, 2]), np.abs((c - ref[:, 1]) - ref[:, 3]))
+        err = sincos_err(s, c, ref)
         off = np.mean(np.concatenate([s != ref[:, 0], c != ref[:, 1]]))  # share of the 2n values
         report[name] = (float(err.max()), float(off))
     print("max abs error, share of values not correctly rounded:", report)
